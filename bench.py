@@ -34,6 +34,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
@@ -47,12 +48,13 @@ FFT_SIZE = 512
 BATCHES_PER_STEP = 8  # one second of signal per input per step
 TEMPLATES = 8         # distinct seeded streams; every input owns a private copy of one of them
 DEPTH = 3             # tickets in flight (the engine has three result slots)
+DUMP_ROWS = 1024      # (input, channel) rows --dump-outputs writes: 1024 x 8000 float32 samples = 32 MB
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of each leg of the headline workload (the other workloads time 4 each)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--inputs", type=int, default=512, help="inputs per GPU")
@@ -62,6 +64,7 @@ def parse_args():
     ap.add_argument("--no-workloads", action="store_true")
     ap.add_argument("--total-inputs", type=int, default=512, help="inputs of the whole job in the strong-scaling leg (N > 1)")
     ap.add_argument("--cpu-seconds", type=float, default=20.0, help="signal seconds per input in the CPU sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of `value` returned as DIR/*.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -132,6 +135,32 @@ def workload_cfg(n_inputs: int, fft_size: int, first_index: int, cuda_device: in
     cfg.cuda_device = cuda_device
     cfg.max_batches_per_step = BATCHES_PER_STEP
     return cfg
+
+
+def dump_outputs(eng, ticket: int, n_inputs: int, out_dir: str):
+    """What ba_cuda_collect returned for `ticket`, so that two builds can be compared output for output on the same seeded
+    inputs.  Rows are (input, channel) pairs: all of them up to DUMP_ROWS, else a fixed seeded sample of DUMP_ROWS.
+      rows.npy    [R, 2] float64   input and channel of each row
+      audio.npy   [R, n] float32   the row's demodulated audio of the step (n = batches x WAVE_BATCH)
+      status.npy  [R, batches, 10] float64   the row's per-batch status: axcindicate, bin, signal, noise and squelch level,
+                                             open, flappy, ctcss and no-ctcss counts, active counter"""
+    os.makedirs(out_dir, exist_ok=True)
+    n_ch = len(eng.cfg.devices[0].channels)
+    total = n_inputs * n_ch
+    rows = np.arange(total) if total <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(total, DUMP_ROWS, replace=False))
+    audio, status = [], []
+    for i in np.unique(rows // n_ch):
+        r = eng.collect(ticket, int(i))
+        for c in rows[rows // n_ch == i] % n_ch:
+            audio.append(r.waveout[c])
+            raw = r.status_raw[:, c, :]
+            st = raw.astype(np.float64)
+            st[:, 0] = raw[:, 0].view(np.int32)
+            st[:, 2:5] = raw[:, 2:5].view(np.float32)
+            status.append(st)
+    np.save(os.path.join(out_dir, "rows.npy"), np.stack([rows // n_ch, rows % n_ch], axis=1).astype(np.float64))
+    np.save(os.path.join(out_dir, "audio.npy"), np.stack(audio).astype(np.float32))
+    np.save(os.path.join(out_dir, "status.npy"), np.stack(status))
 
 
 def host_threads() -> int:
@@ -295,6 +324,8 @@ def main():
     import torch
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes what the GPU path returned: it has no meaning with --impl reference")
         if rank != 0:
             return
         # bounded sample of the same workload on the host cores; templates are made with numpy-free torch CPU ops
@@ -304,13 +335,10 @@ def main():
         vals = []
         for _ in range(max(1, min(W, 1))):
             cpu_reference(args.inputs, args.fft_size, min(1.0, secs), tmpl)
-        t0 = time.time()
         last = None
         for _ in range(K):
             last = cpu_reference(args.inputs, args.fft_size, secs, tmpl)
             vals.append(last["value"])
-            if time.time() - t0 > 150:
-                break
         v = statistics.median(vals)
         line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "Msps", "x_realtime": v * 1e6 / FS, "n_gpus": args.gpus, "steps": len(vals),
                 "warmup": W, "ms_per_step": 1e3 * last["wall_s"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -322,6 +350,8 @@ def main():
 
     from boondock_airband_b200.engine import Engine
 
+    if args.dump_outputs and K < 1:
+        raise SystemExit("--dump-outputs writes the last timed step: it needs --steps 1 or more")
     if world > 1:
         import torch.distributed as dist
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
@@ -352,8 +382,9 @@ def main():
     sampler.start()
     windows = []
 
-    def device_leg(flags, n_inputs=None, first_index=None):
-        """K timed steps with the IQ resident in HBM; flags: where the results go (see the calls below)."""
+    def device_leg(flags, n_inputs=None, first_index=None, dump_dir=None):
+        """K timed steps with the IQ resident in HBM; flags: where the results go (see the calls below); dump_dir: where
+        dump_outputs writes what the last timed step returned."""
         n_in = args.inputs if n_inputs is None else n_inputs
         cfg = workload_cfg(n_in, args.fft_size, sharding.first_input_of_rank(args.inputs, rank) if first_index is None else first_index, local)
         cfg.flags = flags
@@ -363,6 +394,7 @@ def main():
         torch.cuda.synchronize()
         # the first step also has to fill the AGC look-back (B + E frames): hand it a little more than one second
         tickets = []
+        last = [None]
 
         copy_legs = [0.0, 0.0]
         d2h_total = [0]
@@ -376,6 +408,7 @@ def main():
                     eng.advance_device_stream(i, step_bytes + extra)
                 t = eng.process()
                 tickets.append(t)
+                last[0] = t
                 if len(tickets) >= DEPTH:
                     old = tickets.pop(0)
                     r = eng.collect_raw(old, 0)
@@ -407,7 +440,7 @@ def main():
         barrier()
         eng.mark(0)
         t0 = time.perf_counter()
-        k1_ms, k2_ms, batches = run_steps(K, False)
+        k1_ms, k2_ms, batches = run_steps(K, W == 0)
         eng.mark(1)
         barrier()
         t1 = time.perf_counter()
@@ -416,6 +449,8 @@ def main():
         windows.append((t0, t1))
         launches = eng.launch_count() - launches0
         assert batches == K * BATCHES_PER_STEP, "device-resident run produced %d batches, expected %d" % (batches, K * BATCHES_PER_STEP)
+        if dump_dir is not None:
+            dump_outputs(eng, last[0], n_in, dump_dir)
         # timed on the device (CUDA events on the engine's own streams, behind the barrier), max over ranks; the host's wall clock
         # around the same region also contains the closing NCCL barrier and is reported next to it
         elapsed = dev_ms / 1e3
@@ -431,7 +466,7 @@ def main():
     # `value_results_on_device`; the end-to-end leg below has host copies both ways.
     from boondock_airband_b200 import abi as _abi
     leg_dev = device_leg(_abi.FLAG_RESULTS_ON_DEVICE)
-    leg_host = device_leg(0)
+    leg_host = device_leg(0, dump_dir=args.dump_outputs if rank == 0 else None)
     # the same as `value`, but only the (channel, batch) rows that are not silence cross the link (BA_FLAG_SKIP_SILENT_ROWS: decided on
     # the data on the device; the synthetic carriers are keyed 1.5 s on / 0.5 s off, so about a quarter of the rows are silence)
     leg_skip = device_leg(_abi.FLAG_SKIP_SILENT_ROWS)
@@ -501,7 +536,7 @@ def main():
         e2e_legs = [0.0, 0.0, 0.0, 0.0]
         barrier()
         t0 = time.perf_counter()
-        got = e2e_steps(K, False)
+        got = e2e_steps(K, W == 0)
         barrier()
         e2e_wall = time.perf_counter() - t0
         windows.append((t0, t0 + e2e_wall))

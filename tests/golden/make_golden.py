@@ -47,6 +47,7 @@ def pipeline_case(name):
     if iqc:
         out["iq_out"] = np.stack([o.iq_out(0, c) for c in iqc])
         out["iq_channels"] = np.array(iqc)
+    np.savez_compressed(os.path.join(HERE, name + "_iq.npz"), iq=out.pop("iq"))
     np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
     print(name, "frames", out["frames"], "batches", out["batches"], "open samples", int(((out["trace"] & abi.TRACE_OPEN) != 0).sum()))
 

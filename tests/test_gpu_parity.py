@@ -214,9 +214,8 @@ def test_golden_fixtures_on_the_gpu(cuda, name):
     the oracle in between: (1) the stored IQ through the whole engine - bins and decision trace identical, picked-bin IQ
     within 1e-4, audio within 1e-3, counters identical; (2) the stored picked-bin IQ injected behind the channelizer -
     audio, trace and levels bit for bit."""
-    import os
     import golden_cases
-    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name + ".npz"))
+    g = golden_cases.load(name)
     cfg, _ = golden_cases.build(name, with_iq=False)
     nch = len(cfg.devices[0].channels)
     cfg.flags |= abi.FLAG_KEEP_PICKS

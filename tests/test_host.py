@@ -616,13 +616,12 @@ def test_handoff_polling_counts_overruns_like_the_reference():
     L.ba_handoff_destroy(h)
 
 
-def test_host_header_binding_and_exports_agree():
+def test_host_header_binding_and_exports_agree(tmp_path):
     names = sorted(set(re.findall(r"^BA_HOST_API\s+[\w\s\*]+?\b(ba_\w+)\s*\(", open(HEADER).read(), re.M)))
     assert names == sorted(host.SYMBOLS)
     out = subprocess.check_output(["nm", "-D", "--defined-only", host.DEFAULT_LIB], text=True)
     assert set(re.findall(r"\bT (ba_\w+)", out)) == set(names)
     assert "cuda" not in subprocess.check_output(["ldd", host.DEFAULT_LIB], text=True)  # loads on a machine without CUDA
-    src = "/tmp/ba_host_c99_%d.c" % os.getpid()
-    open(src, "w").write('#include "ba_host.h"\nint main(void){return BA_OK;}\n')
-    subprocess.check_call(["gcc", "-std=c99", "-pedantic", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), "-c", "-o", src + ".o", src])
-    os.remove(src), os.remove(src + ".o")
+    src = tmp_path / "ba_host_c99.c"
+    src.write_text('#include "ba_host.h"\nint main(void){return BA_OK;}\n')
+    subprocess.check_call(["gcc", "-std=c99", "-pedantic", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), "-c", "-o", str(tmp_path / "ba_host_c99.o"), str(src)])

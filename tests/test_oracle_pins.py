@@ -274,7 +274,7 @@ def test_golden_dsp_objects(orc):
 @pytest.mark.parametrize("name", golden_cases.NAMES)
 def test_golden_pipeline(orc, name):
     """The restated loop + restated classes reproduce the reference-built oracle's committed outputs bit for bit."""
-    g = np.load(os.path.join(GOLD, name + ".npz"))
+    g = golden_cases.load(name)
     cfg, _ = golden_cases.build(name, with_iq=False)
     o = orc.Oracle(cfg)
     o.feed(0, g["iq"])
@@ -312,6 +312,23 @@ def test_restated_equals_reference_build(orc):
                 assert np.array_equal(a.trace(d, c), b.trace(d, c))
                 sa, sb = a.status(d, c), b.status(d, c)
                 assert [bytes(x) for x in sa] == [bytes(x) for x in sb]
+
+
+@pytest.mark.parametrize("name", sorted(golden_cases.digest_scenarios()))
+def test_oracle_reproduces_recorded_outputs(orc, name):
+    """The scenarios of test_restated_equals_reference_build and of the GPU tests against the reference objects (FM quadri
+    demodulation, cfg2's CTCSS and notch, several inputs, the AGC clip and flapping of am_stress, the AFC walk): the oracle's
+    outputs, bit for bit, against the digests in golden/oracle_digests.json, and the reference-built oracle's too where it exists."""
+    import json
+    with open(os.path.join(GOLD, "oracle_digests.json")) as f:
+        want = json.load(f)[name]
+    cfg, streams = golden_cases.digest_scenarios()[name]()
+    for ref in builds(orc):
+        got = golden_cases.oracle_digests(orc.Oracle, cfg, streams, ref=ref)
+        assert got["inputs"] == want["inputs"], "the scenario's synthesised input is not the recorded one"
+        for key in sorted(want["channels"]):
+            assert got["channels"][key] == want["channels"][key], (ref, key)
+        assert got == want
 
 
 def test_oracle_fft_against_float64_dft(orc):

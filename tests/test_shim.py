@@ -3,6 +3,7 @@ thread body that takes demodulate()'s place, built against include/ba_ref_layout
 (circbuffer_append's arithmetic into the engine's pinned ring, under buffer_lock) and a fake output thread (output.cpp:931-951).
 tests/shim/harness.cpp plays the reference's side; everything it calls in the product goes through the C-ABI."""
 import ctypes as C
+import json
 import os
 import subprocess
 import tempfile
@@ -68,26 +69,31 @@ STUBS = {
 }
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is not mounted here")
 @pytest.mark.parametrize("nfm", [False, True])
 def test_layout_matches_the_reference_headers(nfm):
     """include/ba_ref_layout.h against the reference's own boondock_airband.h (compiled with stub headers in place of lame,
-    shout, libconfig++ and fftw, which are not installed): sizes and the offsets of every member the thread body touches."""
+    shout, libconfig++ and fftw, which are not installed): sizes and the offsets of every member the thread body touches.
+    tests/golden/ref_layout.json holds the probe's output for the reference's header (recorded from include/ba_ref_layout.h
+    at a commit where this test had found the two equal), so the check runs without the reference tree; where the tree is
+    mounted the probe also runs on the reference's header itself."""
+    with open(os.path.join(HERE, "golden", "ref_layout.json")) as f:
+        want = json.load(f)["nfm" if nfm else "am"]
     with tempfile.TemporaryDirectory() as td:
         for rel, text in STUBS.items():
             os.makedirs(os.path.dirname(os.path.join(td, "stubs", rel)), exist_ok=True)
             with open(os.path.join(td, "stubs", rel), "w") as f:
                 f.write(text)
-        outs = []
-        for tag, inc, flags in (("ref", '#include "boondock_airband.h"', ["-I" + os.path.join(td, "stubs"), "-I" + REF]),
-                                ("mine", '#include "ba_ref_layout.h"', ["-I" + os.path.join(ROOT, "include")])):
+        probes = [("mine", '#include "ba_ref_layout.h"', ["-I" + os.path.join(ROOT, "include")])]
+        if os.path.isdir(REF):
+            probes.append(("ref", '#include "boondock_airband.h"', ["-I" + os.path.join(td, "stubs"), "-I" + REF]))
+        for tag, inc, flags in probes:
             src = os.path.join(td, tag + ".cpp")
             with open(src, "w") as f:
                 f.write(PROBE % inc)
             exe = os.path.join(td, tag)
             subprocess.check_call(["g++", "-std=c++14", "-w"] + (["-DNFM"] if nfm else []) + flags + [src, "-o", exe])
-            outs.append(subprocess.check_output([exe]).decode())
-        assert outs[0] == outs[1], "\n" + outs[0] + "---\n" + outs[1]
+            got = subprocess.check_output([exe]).decode()
+            assert got == want, "%s:\n%s---\nreference:\n%s" % (tag, got, want)
 
 
 def test_shim_builds_and_loads_without_a_gpu(shim):
