@@ -61,6 +61,25 @@ int fail(int code, const char* fmt, ...) {
             return fail(BA_ERR_CUDA, "cudaSetDevice(%d) -> %s", (e)->cuda_device, cudaGetErrorString(e_)); \
     } while (0)
 
+/* A group (ba_cuda_create_multi) hands a per-device or per-mixer call to the member that holds that device or mixer, under
+ * the member's own index, and returns what the member returns; `call` is the entry point itself, which then sees a plain
+ * engine. */
+#define FORWARD(e, idx, owner, local, what, call)                                      \
+    do {                                                                                \
+        if ((e) && !(e)->members.empty()) {                                             \
+            ba_engine* g_ = (e);                                                        \
+            if (g_->broken)                                                             \
+                return group_broken();                                                  \
+            if ((idx) < 0 || (idx) >= (int)g_->owner.size())                            \
+                return fail(BA_ERR_BAD_ARG, "no " what " %d", (int)(idx));              \
+            e = g_->members[g_->owner[idx]];                                            \
+            idx = g_->local[idx];                                                       \
+            return group_rc(g_, (call));                                                \
+        }                                                                               \
+    } while (0)
+#define FORWARD_DEV(e, dev, call) FORWARD(e, dev, dev_member, dev_local, "device", call)
+#define FORWARD_MIXER(e, mixer, call) FORWARD(e, mixer, mix_member, mix_local, "mixer", call)
+
 uint32_t pow2_at_least(uint64_t v) {
     uint32_t p = 1;
     while (p < v)
@@ -234,6 +253,11 @@ struct ba_engine {
     int fifo_depth = 0;
     size_t mix_floats = 0;   /* floats of one slot's mixer arena */
     size_t mix_desc_off = 0; /* where the K3 part of the per-ticket descriptor blob starts */
+    /* ba_cuda_create_multi(): a group holds nothing but its members (ordinary engines) and where each device and mixer went */
+    std::vector<ba_engine*> members;
+    std::vector<int> dev_member, dev_local; /* per device of the group's descriptor */
+    std::vector<int> mix_member, mix_local; /* per mixer */
+    bool broken = false;                    /* a member failed in a way that may leave the members out of step */
 };
 
 namespace {
@@ -241,6 +265,12 @@ namespace {
 void free_engine(ba_engine* e) {
     if (!e)
         return;
+    if (!e->members.empty()) {
+        for (ba_engine* m : e->members)
+            free_engine(m);
+        delete e;
+        return;
+    }
     cudaSetDevice(e->cuda_device);
     for (cudaStream_t q : {e->s_in, e->s_in2, e->s_k, e->s_k2, e->s_k2b, e->s_out, e->s_pack})
         if (q)
@@ -336,6 +366,45 @@ void free_engine(ba_engine* e) {
         if (ev)
             cudaEventDestroy(ev);
     delete e;
+}
+
+/* A member's error that may have left it out of step with the others (a CUDA failure, a half-made pass) ends the group's
+ * useful life; refusals (bad arguments, a full ring, a call out of sequence) change nothing and are just returned. */
+int group_rc(ba_engine* g, int rc) {
+    if (rc == BA_ERR_CUDA || rc == BA_ERR_NOMEM)
+        g->broken = true;
+    return rc;
+}
+
+int group_broken() {
+    return fail(BA_ERR_STATE, "a member of this multi-GPU engine failed; the handle is only good for ba_cuda_destroy()");
+}
+
+/* Runs f on every member of a group in member order; stops at the first error. */
+template <class F>
+int each_member(ba_engine* g, F f) {
+    if (g->broken)
+        return group_broken();
+    for (ba_engine* m : g->members) {
+        const int rc = group_rc(g, f(m));
+        if (rc < 0)
+            return rc;
+    }
+    return BA_OK;
+}
+
+/* For the per-ticket timings that come in pairs: each element is the maximum over the members. */
+int max_pair_over_members(ba_engine* g, int ticket, float ms[2], int (*get)(ba_engine*, int, float*)) {
+    if (!ms)
+        return fail(BA_ERR_BAD_ARG, "null argument");
+    ms[0] = ms[1] = 0.0f;
+    return each_member(g, [&](ba_engine* m) {
+        float v[2] = {0.0f, 0.0f};
+        const int r = get(m, ticket, v);
+        ms[0] = std::max(ms[0], v[0]);
+        ms[1] = std::max(ms[1], v[1]);
+        return r;
+    });
 }
 
 /* frames the reference's availability test admits for a stream of `total` bytes (.cpp:418-424 with FFT_BATCH 1):
@@ -921,6 +990,138 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
     return BA_OK;
 }
 
+int ba_cuda_create_multi(const ba_engine_desc* desc, const int32_t* gpus, int32_t n_gpus, const int32_t* gpu_of_device, ba_engine** out) {
+    if (!desc || !out || !gpus)
+        return fail(BA_ERR_BAD_ARG, "null argument");
+    *out = nullptr;
+    if (n_gpus < 1)
+        return fail(BA_ERR_BAD_ARG, "n_gpus %d: a multi-GPU engine needs at least one GPU", n_gpus);
+    const int nd = desc->device_count, n_mixers = desc->mixer_count;
+    if (nd <= 0 || !desc->devices)
+        return fail(BA_ERR_BAD_ARG, "no devices");
+    if (n_mixers < 0 || (n_mixers > 0 && !desc->mixers))
+        return fail(BA_ERR_BAD_ARG, "mixer_count %d without mixers", n_mixers);
+    int visible = 0;
+    cudaError_t ce = cudaGetDeviceCount(&visible);
+    if (ce != cudaSuccess || visible <= 0)
+        return fail(BA_ERR_NO_DEVICE, "no CUDA device (%s); this engine has no CPU path", ce != cudaSuccess ? cudaGetErrorString(ce) : "count 0");
+    for (int k = 0; k < n_gpus; k++)
+        if (gpus[k] < 0 || gpus[k] >= visible)
+            return fail(BA_ERR_BAD_ARG, "gpus[%d] = %d is not a visible CUDA device (%d visible)", k, gpus[k], visible);
+    for (int m = 0; m < n_mixers; m++) {
+        const ba_mixer_desc& md = desc->mixers[m];
+        if (md.input_count < 0 || (md.input_count > 0 && !md.inputs))
+            return fail(BA_ERR_BAD_ARG, "mixer %d: bad input list", m);
+        for (int j = 0; j < md.input_count; j++)
+            if (md.inputs[j].device < 0 || md.inputs[j].device >= nd)
+                return fail(BA_ERR_BAD_ARG, "mixer %d input %d: no device %d", m, j, md.inputs[j].device);
+    }
+    /* which entry of gpus every device goes to */
+    std::vector<int> where(nd);
+    if (gpu_of_device) {
+        for (int d = 0; d < nd; d++) {
+            if (gpu_of_device[d] < 0 || gpu_of_device[d] >= n_gpus)
+                return fail(BA_ERR_BAD_ARG, "gpu_of_device[%d] = %d is not an index into the %d gpus", d, gpu_of_device[d], n_gpus);
+            where[d] = gpu_of_device[d];
+        }
+        for (int m = 0; m < n_mixers; m++) {
+            const ba_mixer_desc& md = desc->mixers[m];
+            for (int j = 1; j < md.input_count; j++)
+                if (where[md.inputs[j].device] != where[md.inputs[0].device])
+                    return fail(BA_ERR_BAD_ARG, "mixer %d has inputs on gpus[%d] and gpus[%d]; a mixer's inputs must share one GPU", m,
+                                where[md.inputs[0].device], where[md.inputs[j].device]);
+        }
+    } else {
+        /* devices joined by a mixer form one group (union-find, each set rooted at its first device); groups are dealt out
+         * round robin in the order of their first device */
+        std::vector<int> root(nd);
+        for (int d = 0; d < nd; d++)
+            root[d] = d;
+        auto find = [&](int d) {
+            while (root[d] != d)
+                d = root[d] = root[root[d]];
+            return d;
+        };
+        for (int m = 0; m < n_mixers; m++) {
+            const ba_mixer_desc& md = desc->mixers[m];
+            for (int j = 1; j < md.input_count; j++) {
+                const int a = find(md.inputs[0].device), b = find(md.inputs[j].device);
+                root[std::max(a, b)] = std::min(a, b);
+            }
+        }
+        std::vector<int> group_of_root(nd, -1);
+        int groups = 0;
+        for (int d = 0; d < nd; d++) {
+            const int r = find(d);
+            if (group_of_root[r] < 0)
+                group_of_root[r] = groups++;
+            where[d] = group_of_root[r] % n_gpus;
+        }
+    }
+
+    ba_engine* g = new (std::nothrow) ba_engine();
+    if (!g)
+        return fail(BA_ERR_NOMEM, "host allocation");
+    g->dev_member.assign(nd, -1);
+    g->dev_local.assign(nd, -1);
+    g->mix_member.assign(n_mixers, -1);
+    g->mix_local.assign(n_mixers, -1);
+    /* one member per entry of gpus that received devices, in the order of gpus; a mixer without inputs goes with device 0 */
+    for (int k = 0; k < n_gpus; k++) {
+        std::vector<ba_device_desc> devs;
+        for (int d = 0; d < nd; d++)
+            if (where[d] == k) {
+                g->dev_member[d] = (int)g->members.size();
+                g->dev_local[d] = (int)devs.size();
+                devs.push_back(desc->devices[d]);
+            }
+        if (devs.empty())
+            continue;
+        std::vector<ba_mixer_desc> mixers;
+        std::vector<std::vector<ba_mixer_input_desc>> inputs;
+        for (int m = 0; m < n_mixers; m++) {
+            const ba_mixer_desc& md = desc->mixers[m];
+            if ((md.input_count > 0 ? where[md.inputs[0].device] : where[0]) != k)
+                continue;
+            g->mix_member[m] = (int)g->members.size();
+            g->mix_local[m] = (int)mixers.size();
+            inputs.emplace_back(md.inputs, md.inputs + md.input_count);
+            for (ba_mixer_input_desc& in : inputs.back())
+                in.device = g->dev_local[in.device];
+            mixers.push_back(ba_mixer_desc{md.input_count, nullptr});
+        }
+        for (size_t m = 0; m < mixers.size(); m++)
+            mixers[m].inputs = inputs[m].data();
+        ba_engine_desc sub = *desc;
+        sub.cuda_device = gpus[k];
+        sub.device_count = (int32_t)devs.size();
+        sub.devices = devs.data();
+        sub.mixer_count = (int32_t)mixers.size();
+        sub.mixers = mixers.empty() ? nullptr : mixers.data();
+        ba_engine* m = nullptr;
+        const int rc = ba_cuda_create(&sub, &m);
+        if (rc != BA_OK) {
+            for (ba_engine* x : g->members)
+                free_engine(x);
+            delete g;
+            return rc;
+        }
+        g->members.push_back(m);
+    }
+    *out = g;
+    return BA_OK;
+}
+
+int ba_cuda_device_gpu(ba_engine* e, int dev, int32_t* cuda_ordinal) {
+    if (!cuda_ordinal)
+        return fail(BA_ERR_BAD_ARG, "null argument");
+    FORWARD_DEV(e, dev, ba_cuda_device_gpu(e, dev, cuda_ordinal));
+    if (!e || dev < 0 || dev >= (int)e->dev.size())
+        return fail(BA_ERR_BAD_ARG, "bad engine or device index %d", dev);
+    *cuda_ordinal = e->cuda_device;
+    return BA_OK;
+}
+
 static Dev* get_dev(ba_engine* e, int dev) {
     if (!e || dev < 0 || dev >= (int)e->dev.size()) {
         fail(BA_ERR_BAD_ARG, "bad engine or device index %d", dev);
@@ -930,6 +1131,7 @@ static Dev* get_dev(ba_engine* e, int dev) {
 }
 
 int ba_cuda_input_ring(ba_engine* e, int dev, unsigned char** buffer, size_t* buf_size, size_t* mirror_bytes) {
+    FORWARD_DEV(e, dev, ba_cuda_input_ring(e, dev, buffer, buf_size, mirror_bytes));
     Dev* d = get_dev(e, dev);
     if (!d)
         return BA_ERR_BAD_ARG;
@@ -984,6 +1186,7 @@ static bool ring_release_pending(ba_engine* e, cudaEvent_t ev) {
 }
 
 int ba_cuda_submit(ba_engine* e, int dev, const void* iq, size_t len) {
+    FORWARD_DEV(e, dev, ba_cuda_submit(e, dev, iq, len));
     Dev* d = get_dev(e, dev);
     if (!d || (!iq && len))
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1016,6 +1219,7 @@ int ba_cuda_submit(ba_engine* e, int dev, const void* iq, size_t len) {
 }
 
 int ba_cuda_input_space(ba_engine* e, int dev, size_t* free_bytes) {
+    FORWARD_DEV(e, dev, ba_cuda_input_space(e, dev, free_bytes));
     Dev* d = get_dev(e, dev);
     if (!d || !free_bytes)
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1028,6 +1232,7 @@ int ba_cuda_input_space(ba_engine* e, int dev, size_t* free_bytes) {
 }
 
 int ba_cuda_commit(ba_engine* e, int dev, size_t len) {
+    FORWARD_DEV(e, dev, ba_cuda_commit(e, dev, len));
     Dev* d = get_dev(e, dev);
     if (!d)
         return BA_ERR_BAD_ARG;
@@ -1046,6 +1251,7 @@ int ba_cuda_commit(ba_engine* e, int dev, size_t len) {
 }
 
 int ba_cuda_input_consumed(ba_engine* e, int dev, size_t* bufs) {
+    FORWARD_DEV(e, dev, ba_cuda_input_consumed(e, dev, bufs));
     Dev* d = get_dev(e, dev);
     if (!d || !bufs)
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1056,6 +1262,7 @@ int ba_cuda_input_consumed(ba_engine* e, int dev, size_t* bufs) {
 }
 
 int ba_cuda_submit_external(ba_engine* e, int dev, const void* iq, size_t len) {
+    FORWARD_DEV(e, dev, ba_cuda_submit_external(e, dev, iq, len));
     Dev* d = get_dev(e, dev);
     if (!d || (!iq && len))
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1071,6 +1278,7 @@ int ba_cuda_submit_external(ba_engine* e, int dev, const void* iq, size_t len) {
 }
 
 int ba_cuda_attach_device_stream(ba_engine* e, int dev, const void* d_iq, size_t capacity_bytes) {
+    FORWARD_DEV(e, dev, ba_cuda_attach_device_stream(e, dev, d_iq, capacity_bytes));
     Dev* d = get_dev(e, dev);
     if (!d || !d_iq)
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1085,6 +1293,7 @@ int ba_cuda_attach_device_stream(ba_engine* e, int dev, const void* d_iq, size_t
 }
 
 int ba_cuda_advance_device_stream(ba_engine* e, int dev, size_t bytes) {
+    FORWARD_DEV(e, dev, ba_cuda_advance_device_stream(e, dev, bytes));
     Dev* d = get_dev(e, dev);
     if (!d)
         return BA_ERR_BAD_ARG;
@@ -1112,6 +1321,19 @@ static uint64_t frame_room(const ba_engine* e, const Dev& d) {
 }
 
 int ba_cuda_process(ba_engine* e) {
+    if (e && !e->members.empty()) { /* every member's pass; their tickets move in lockstep */
+        int ticket = -1;
+        const int rc = each_member(e, [&](ba_engine* m) {
+            const int t = ba_cuda_process(m);
+            if (t >= 0 && ticket >= 0 && t != ticket)
+                return fail(BA_ERR_STATE, "member tickets %d and %d differ", ticket, t);
+            ticket = t;
+            return t;
+        });
+        if (rc < 0)
+            e->broken = true;
+        return rc < 0 ? rc : ticket;
+    }
     using namespace ba;
     if (!e)
         return fail(BA_ERR_BAD_ARG, "null engine");
@@ -1271,9 +1493,17 @@ int ba_cuda_process(ba_engine* e) {
     K2Dyn* h_dyn = reinterpret_cast<K2Dyn*>(s.h_desc + (size_t)e->max_phases * nd * sizeof(K1Device));
     K1Device* d_k1 = reinterpret_cast<K1Device*>(s.d_desc);
     K2Dyn* d_dyn = reinterpret_cast<K2Dyn*>(s.d_desc + (size_t)e->max_phases * nd * sizeof(K1Device));
-    std::vector<int> k1_count(phases, 0), k1_tiles(phases, 0), k2_any(phases, 0);
+    /* K1 entries of a phase: inputs without AFC first, then the AFC inputs, which need the instantiation that also writes the
+     * spectrum (k1_plain / k1_plain_tiles: entries and tiles of the first kind); each kind is one launch */
+    std::vector<int> k1_count(phases, 0), k1_tiles(phases, 0), k2_any(phases, 0), k1_plain(phases, 0), k1_plain_tiles(phases, 0);
+    std::vector<size_t> order;
+    for (int afc = 0; afc < 2; afc++)
+        for (size_t di = 0; di < nd; di++)
+            if (e->dev[di]->any_afc == (afc == 1))
+                order.push_back(di);
     for (int ph = 0; ph < phases; ph++) {
-        for (size_t di = 0; di < nd; di++) {
+        for (size_t oi = 0; oi < nd; oi++) {
+            const size_t di = order[oi];
             Dev& d = *e->dev[di];
             uint64_t f_begin, f_end;
             int nb_here, b_first;
@@ -1309,13 +1539,18 @@ int ba_cuda_process(ba_engine* e) {
                 k.mags = d.d_mags;
                 k.ring_mask = d.ring_len - 1;
                 k.n_channels = (uint32_t)d.C;
-                k.tile0 = (uint32_t)k1_tiles[ph];
+                k.tile0 = (uint32_t)(k1_tiles[ph] - (d.any_afc ? k1_plain_tiles[ph] : 0)); /* tiles count from 0 in each launch */
                 k.bins = d.d_bins;
                 k.scale = 1.0f / d.cfg.fullscale;
                 k.fmt = d.cfg.sample_format;
                 k.spectrum = (d.any_afc && nb_here) ? d.d_spectrum : nullptr;
-                k1_tiles[ph] += (int)((k.n_frames + e->tile_frames - 1) / e->tile_frames);
+                const int tiles = (int)((k.n_frames + e->tile_frames - 1) / e->tile_frames);
+                k1_tiles[ph] += tiles;
                 k1_count[ph]++;
+                if (!d.any_afc) {
+                    k1_plain[ph]++;
+                    k1_plain_tiles[ph] += tiles;
+                }
             }
             K2Dyn& y = h_dyn[(size_t)ph * nd + di];
             memset(&y, 0, sizeof(y));
@@ -1396,12 +1631,19 @@ int ba_cuda_process(ba_engine* e) {
     cudaStream_t k2s = e->serial_k2 ? e->s_k : e->s_k2;
     for (int ph = 0; ph < phases; ph++) {
         CU(cudaEventRecord(s.ev_k[4 * ph + 0], e->s_k));
-        if (k1_count[ph]) {
+        /* Inputs without AFC never run the instantiation that also writes the spectrum: the two are compiled apart and may
+         * round the FFT differently in the last bit, and an input's audio must not depend on whether another input of its
+         * engine has AFC (nor on which member of a multi-GPU group it was placed in). */
+        for (int afc = 0; afc < 2; afc++) {
+            const int first = afc ? k1_plain[ph] : 0;
+            const int n_dev = afc ? k1_count[ph] - k1_plain[ph] : k1_plain[ph];
+            if (n_dev == 0)
+                continue;
             K1Params p;
-            p.dev = d_k1 + (size_t)ph * nd;
-            p.n_dev = k1_count[ph];
+            p.dev = d_k1 + (size_t)ph * nd + first;
+            p.n_dev = n_dev;
             p.tile_frames = e->tile_frames;
-            p.n_tiles = k1_tiles[ph];
+            p.n_tiles = afc ? k1_tiles[ph] - k1_plain_tiles[ph] : k1_plain_tiles[ph];
             p.window = e->d_window;
             p.twiddle = e->d_twiddle;
             p.raw_bytes = e->raw_bytes;
@@ -1409,7 +1651,7 @@ int ba_cuda_process(ba_engine* e) {
             p.tile_counter = e->d_tile_counter;
             const int ctas = std::min(p.n_tiles, e->sm_count * e->k1_ctas_per_sm);
             CU(cudaMemsetAsync(e->d_tile_counter, 0, sizeof(uint32_t), e->s_k));
-            int rc = k1_launch(e->fft_size, p, ctas, e->any_afc, e->s_k);
+            int rc = k1_launch(e->fft_size, p, ctas, afc != 0, e->s_k);
             if (rc != 0)
                 return fail(BA_ERR_CUDA, "channelize launch: %s", cudaGetErrorString((cudaError_t)rc));
             e->launches++;
@@ -1597,6 +1839,7 @@ static Slot* find_slot(ba_engine* e, int ticket) {
 }
 
 int ba_cuda_collect(ba_engine* e, int ticket, int dev, ba_step_out* out) {
+    FORWARD_DEV(e, dev, ba_cuda_collect(e, ticket, dev, out));
     Slot* s = find_slot(e, ticket);
     Dev* d = get_dev(e, dev);
     if (!s || !d || !out)
@@ -1636,6 +1879,7 @@ int ba_cuda_collect(ba_engine* e, int ticket, int dev, ba_step_out* out) {
 }
 
 int ba_cuda_collect_mixer(ba_engine* e, int ticket, int mixer, ba_mixer_out* out) {
+    FORWARD_MIXER(e, mixer, ba_cuda_collect_mixer(e, ticket, mixer, out));
     Slot* s = find_slot(e, ticket);
     if (!s)
         return BA_ERR_BAD_ARG;
@@ -1657,6 +1901,7 @@ int ba_cuda_collect_mixer(ba_engine* e, int ticket, int mixer, ba_mixer_out* out
 }
 
 int ba_cuda_mixer_input_mask(ba_engine* e, int mixer, int input, int enabled) {
+    FORWARD_MIXER(e, mixer, ba_cuda_mixer_input_mask(e, mixer, input, enabled));
     if (!e || mixer < 0 || mixer >= (int)e->mixers.size() || input < 0 || input >= e->mixers[mixer].n_in)
         return fail(BA_ERR_BAD_ARG, "no input %d on mixer %d", input, mixer);
     MixInput& mi = e->mix_in[e->mixers[mixer].first_in + input];
@@ -1667,6 +1912,7 @@ int ba_cuda_mixer_input_mask(ba_engine* e, int mixer, int input, int enabled) {
 }
 
 int ba_cuda_set_freq_idx(ba_engine* e, int dev, int channel, int freq_idx, uint64_t* from_batch) {
+    FORWARD_DEV(e, dev, ba_cuda_set_freq_idx(e, dev, channel, freq_idx, from_batch));
     Dev* d = get_dev(e, dev);
     if (!d)
         return BA_ERR_BAD_ARG;
@@ -1691,6 +1937,19 @@ int ba_cuda_set_freq_idx(ba_engine* e, int dev, int channel, int freq_idx, uint6
 }
 
 int ba_cuda_ticket_ms(ba_engine* e, int ticket, float* ms) {
+    if (e && !e->members.empty()) {
+        if (!ms)
+            return fail(BA_ERR_BAD_ARG, "null argument");
+        float worst = 0.0f;
+        const int rc = each_member(e, [&](ba_engine* m) {
+            float v = 0.0f;
+            const int r = ba_cuda_ticket_ms(m, ticket, &v);
+            worst = std::max(worst, v);
+            return r;
+        });
+        *ms = worst;
+        return rc;
+    }
     Slot* s = find_slot(e, ticket);
     if (!s || !ms)
         return BA_ERR_BAD_ARG;
@@ -1701,6 +1960,8 @@ int ba_cuda_ticket_ms(ba_engine* e, int ticket, float* ms) {
 }
 
 int ba_cuda_kernel_ms(ba_engine* e, int ticket, float ms[2]) {
+    if (e && !e->members.empty())
+        return max_pair_over_members(e, ticket, ms, ba_cuda_kernel_ms);
     Slot* s = find_slot(e, ticket);
     if (!s || !ms)
         return BA_ERR_BAD_ARG;
@@ -1718,6 +1979,8 @@ int ba_cuda_kernel_ms(ba_engine* e, int ticket, float ms[2]) {
 }
 
 int ba_cuda_copy_ms(ba_engine* e, int ticket, float ms[2]) {
+    if (e && !e->members.empty())
+        return max_pair_over_members(e, ticket, ms, ba_cuda_copy_ms);
     Slot* s = find_slot(e, ticket);
     if (!s || !ms)
         return BA_ERR_BAD_ARG;
@@ -1729,6 +1992,20 @@ int ba_cuda_copy_ms(ba_engine* e, int ticket, float ms[2]) {
 }
 
 int ba_cuda_step_bytes(ba_engine* e, int ticket, uint64_t* h2d, uint64_t* d2h) {
+    if (e && !e->members.empty()) {
+        uint64_t sum[2] = {0, 0};
+        const int rc = each_member(e, [&](ba_engine* m) {
+            uint64_t a = 0, b = 0;
+            const int r = ba_cuda_step_bytes(m, ticket, &a, &b);
+            sum[0] += a, sum[1] += b;
+            return r;
+        });
+        if (h2d)
+            *h2d = sum[0];
+        if (d2h)
+            *d2h = sum[1];
+        return rc;
+    }
     Slot* s = find_slot(e, ticket);
     if (!s)
         return BA_ERR_BAD_ARG;
@@ -1740,6 +2017,8 @@ int ba_cuda_step_bytes(ba_engine* e, int ticket, uint64_t* h2d, uint64_t* d2h) {
 }
 
 int ba_cuda_mark(ba_engine* e, int which) {
+    if (e && !e->members.empty())
+        return each_member(e, [&](ba_engine* m) { return ba_cuda_mark(m, which); });
     if (!e || which < 0 || which >= 8)
         return fail(BA_ERR_BAD_ARG, "bad mark %d", which);
     USE_DEVICE(e);
@@ -1754,6 +2033,19 @@ int ba_cuda_mark(ba_engine* e, int which) {
 }
 
 int ba_cuda_mark_ms(ba_engine* e, int from, int to, float* ms) {
+    if (e && !e->members.empty()) {
+        if (!ms)
+            return fail(BA_ERR_BAD_ARG, "null argument");
+        float worst = 0.0f;
+        const int rc = each_member(e, [&](ba_engine* m) {
+            float v = 0.0f;
+            const int r = ba_cuda_mark_ms(m, from, to, &v);
+            worst = std::max(worst, v);
+            return r;
+        });
+        *ms = worst;
+        return rc;
+    }
     if (!e || !ms || from < 0 || from >= 8 || to < 0 || to >= 8 || !e->marks[from] || !e->marks[to])
         return fail(BA_ERR_BAD_ARG, "marks %d, %d not recorded", from, to);
     USE_DEVICE(e);
@@ -1764,6 +2056,7 @@ int ba_cuda_mark_ms(ba_engine* e, int from, int to, float* ms) {
 }
 
 int ba_cuda_channel_info(ba_engine* e, int dev, int channel, ba_channel_info* out) {
+    FORWARD_DEV(e, dev, ba_cuda_channel_info(e, dev, channel, out));
     Dev* d = get_dev(e, dev);
     if (!d || !out || channel < 0 || channel >= d->C)
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1772,6 +2065,8 @@ int ba_cuda_channel_info(ba_engine* e, int dev, int channel, ba_channel_info* ou
 }
 
 int ba_cuda_window(ba_engine* e, float* out, size_t count) {
+    if (e && !e->members.empty()) /* every member computed the same window */
+        return e->broken ? group_broken() : ba_cuda_window(e->members[0], out, count);
     if (!e || !out || count != e->window.size())
         return fail(BA_ERR_BAD_ARG, "bad argument");
     memcpy(out, e->window.data(), count * sizeof(float));
@@ -1779,6 +2074,19 @@ int ba_cuda_window(ba_engine* e, float* out, size_t count) {
 }
 
 int ba_cuda_launch_count(ba_engine* e, uint64_t* launches) {
+    if (e && !e->members.empty()) {
+        if (!launches)
+            return fail(BA_ERR_BAD_ARG, "null argument");
+        uint64_t sum = 0;
+        const int rc = each_member(e, [&](ba_engine* m) {
+            uint64_t n = 0;
+            const int r = ba_cuda_launch_count(m, &n);
+            sum += n;
+            return r;
+        });
+        *launches = sum;
+        return rc;
+    }
     if (!e || !launches)
         return fail(BA_ERR_BAD_ARG, "bad argument");
     *launches = e->launches;
@@ -1786,6 +2094,7 @@ int ba_cuda_launch_count(ba_engine* e, uint64_t* launches) {
 }
 
 int ba_cuda_debug_frames(ba_engine* e, int dev, const void* iq, size_t bytes, int n_frames, float* fftin, float* fftout) {
+    FORWARD_DEV(e, dev, ba_cuda_debug_frames(e, dev, iq, bytes, n_frames, fftin, fftout));
     using namespace ba;
     Dev* d = get_dev(e, dev);
     if (!d || !iq || n_frames <= 0)
@@ -1870,6 +2179,7 @@ int ba_cuda_debug_frames(ba_engine* e, int dev, const void* iq, size_t bytes, in
 }
 
 int ba_cuda_debug_picks(ba_engine* e, int dev, int channel, uint64_t first, int count, float* out) {
+    FORWARD_DEV(e, dev, ba_cuda_debug_picks(e, dev, channel, first, count, out));
     Dev* d = get_dev(e, dev);
     if (!d || !out || channel < 0 || channel >= d->C || count < 0)
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -1895,6 +2205,7 @@ int ba_cuda_debug_picks(ba_engine* e, int dev, int channel, uint64_t first, int 
 }
 
 int ba_cuda_debug_inject_picks(ba_engine* e, int dev, const float* picks, int n_frames) {
+    FORWARD_DEV(e, dev, ba_cuda_debug_inject_picks(e, dev, picks, n_frames));
     Dev* d = get_dev(e, dev);
     if (!d || !picks || n_frames < 0)
         return fail(BA_ERR_BAD_ARG, "bad argument");

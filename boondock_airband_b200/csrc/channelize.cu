@@ -24,6 +24,10 @@
  */
 #include <stdint.h>
 
+#include <map>
+#include <mutex>
+#include <utility>
+
 #include "ba_kernels.h"
 #include "ba_f32x2.h"
 
@@ -703,9 +707,9 @@ int launch_n(const K1Params& p, int n_ctas, cudaStream_t s) {
     return (int)cudaGetLastError();
 }
 
-/* The dynamic shared-memory limit of a kernel is an attribute of the (device, function) pair: the engine sets it once per
- * engine, right after cudaSetDevice() in ba_cuda_create(), for both instantiations it may launch on that device - never
- * through a process-wide flag (one process may drive one engine per GPU, boondock_airband.cpp:1088-1122). */
+/* The dynamic shared-memory limit of a kernel is an attribute of the (device, function) pair: it is set per device, right
+ * after cudaSetDevice() in ba_cuda_create(), for both instantiations an engine may launch there - never through a
+ * process-wide flag (one process may drive one engine per GPU, boondock_airband.cpp:1088-1122). */
 template <int N>
 int configure_n(size_t smem) {
     cudaError_t e;
@@ -787,17 +791,32 @@ int k1_smem_bytes(int n, int raw_bytes, int max_channels) {
 /* sizes whose frames are read straight from global memory: no tile staging, raw_bytes = 0 */
 int k1_direct(int n) { return n == 8192 ? 1 : 0; }
 
+/* Engines on one GPU share the attribute: one that needs less must not lower it under another's launches, so the limit
+ * set per (device, FFT size) only ever goes up. */
 int k1_configure(int fft_size, int raw_bytes, int max_channels) {
+    static std::mutex lock;
+    static std::map<std::pair<int, int>, size_t> limit;
     const size_t smem = (size_t)k1_smem_bytes(fft_size, raw_bytes, max_channels);
+    int device = 0;
+    cudaError_t e = cudaGetDevice(&device);
+    if (e != cudaSuccess)
+        return (int)e;
+    std::lock_guard<std::mutex> g(lock);
+    size_t& have = limit[std::make_pair(device, fft_size)];
+    if (smem <= have)
+        return 0;
+    int rc = (int)cudaErrorInvalidValue;
     switch (fft_size) {
-        case 256: return configure_n<256>(smem);
-        case 512: return configure_n<512>(smem);
-        case 1024: return configure_n<1024>(smem);
-        case 2048: return configure_n<2048>(smem);
-        case 4096: return configure_n<4096>(smem);
-        case 8192: return configure_n<8192>(smem);
+        case 256: rc = configure_n<256>(smem); break;
+        case 512: rc = configure_n<512>(smem); break;
+        case 1024: rc = configure_n<1024>(smem); break;
+        case 2048: rc = configure_n<2048>(smem); break;
+        case 4096: rc = configure_n<4096>(smem); break;
+        case 8192: rc = configure_n<8192>(smem); break;
     }
-    return (int)cudaErrorInvalidValue;
+    if (rc == 0)
+        have = smem;
+    return rc;
 }
 
 int k1_launch(int fft_size, const K1Params& p, int n_ctas, bool dbg, cudaStream_t s) {

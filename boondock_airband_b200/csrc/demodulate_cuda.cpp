@@ -28,6 +28,7 @@ extern enum fm_demod_algo fm_demod;
 
 #include <math.h>
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
 #include <unistd.h>
 
@@ -53,6 +54,31 @@ int max_batches_from_env() {
     const char* s = getenv("BA_CUDA_MAX_BATCHES");
     const int v = s ? atoi(s) : 1;
     return v < 1 ? 1 : (v > 64 ? 64 : v);
+}
+
+/* BA_CUDA_DEVICES: the GPUs the demodulator threads use.  Unset: GPU 0 alone (empty list).  "all": every visible GPU.
+ * "0,2,3": those CUDA ordinals.  False on anything else. */
+bool gpus_from_env(std::vector<int32_t>& gpus) {
+    gpus.clear();
+    const char* s = getenv("BA_CUDA_DEVICES");
+    if (!s)
+        return true;
+    if (!strcmp(s, "all")) {
+        const int n = ba_cuda_visible_devices();
+        for (int i = 0; i < n; i++)
+            gpus.push_back(i);
+        return n > 0;
+    }
+    for (;;) {
+        char* end;
+        const long v = strtol(s, &end, 10);
+        if (end == s || v < 0 || v > 1023 || (*end != ',' && *end != 0))
+            return false;
+        gpus.push_back((int32_t)v);
+        if (*end == 0)
+            return true;
+        s = end + 1;
+    }
 }
 
 void describe(int devno, device_t* dev, ba_device_desc* d, std::vector<ba_channel_desc>& ch) {
@@ -107,10 +133,25 @@ void* demodulate_cuda(void* params) { /* void* demodulate(void* params), boondoc
     ed.max_batches_per_step = max_batches_from_env();
     if (getenv("BA_CUDA_SKIP_SILENT_ROWS")) /* replays far above real time: silence does not cross the link (see ba_cuda.h) */
         ed.flags |= BA_FLAG_SKIP_SILENT_ROWS;
+    std::vector<int32_t> gpus;
+    if (!gpus_from_env(gpus)) {
+        fprintf(stderr, "BA_CUDA_DEVICES=%s: expected \"all\" or a comma-separated list of CUDA ordinals\n", getenv("BA_CUDA_DEVICES"));
+        do_exit = 1;
+        return NULL;
+    }
+    /* a thread of several devices (the reference's default: one thread for all) spreads them over the GPUs as one engine;
+     * a thread of one device (multiple_demod_threads) takes the GPU its first device number picks from the list */
     ba_engine* eng = NULL;
-    const int ret = ba_cuda_create(&ed, &eng);
+    int ret;
+    if (gpus.empty() || n == 1) {
+        if (!gpus.empty())
+            ed.cuda_device = gpus[first % gpus.size()];
+        ret = ba_cuda_create(&ed, &eng);
+    } else {
+        ret = ba_cuda_create_multi(&ed, gpus.data(), (int32_t)gpus.size(), NULL, &eng);
+    }
     if (ret != BA_OK) { /* the reference's reaction to a failing gpu_fft_prepare(), boondock_airband.cpp:319-332 */
-        fprintf(stderr, "ba_cuda_create: %d (%s)\n", ret, ba_cuda_last_error());
+        fprintf(stderr, "%s: %d (%s)\n", gpus.size() > 0 && n > 1 ? "ba_cuda_create_multi" : "ba_cuda_create", ret, ba_cuda_last_error());
         do_exit = 1;
         return NULL;
     }

@@ -12,7 +12,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import List, Optional
+from typing import List, Optional, Sequence
 
 import numpy as np
 
@@ -30,6 +30,7 @@ SYMBOLS = (
     "ba_cuda_advance_device_stream", "ba_cuda_process", "ba_cuda_collect", "ba_cuda_collect_mixer", "ba_cuda_mixer_input_mask", "ba_cuda_set_freq_idx", "ba_cuda_ticket_ms", "ba_cuda_step_bytes",
     "ba_cuda_channel_info", "ba_cuda_window", "ba_cuda_debug_frames", "ba_cuda_debug_picks",
     "ba_cuda_debug_inject_picks", "ba_cuda_launch_count", "ba_cuda_kernel_ms", "ba_cuda_copy_ms", "ba_cuda_mark", "ba_cuda_mark_ms",
+    "ba_cuda_create_multi", "ba_cuda_device_gpu",
 )
 
 
@@ -50,6 +51,9 @@ def load_library(path: Optional[str] = None):
     L = C.CDLL(path)
     vp, sz, u64p = C.c_void_p, C.c_size_t, C.POINTER(C.c_uint64)
     L.ba_cuda_create.argtypes = [C.POINTER(abi.EngineDesc), C.POINTER(vp)]
+    i32p = C.POINTER(C.c_int32)
+    L.ba_cuda_create_multi.argtypes = [C.POINTER(abi.EngineDesc), i32p, C.c_int32, i32p, C.POINTER(vp)]
+    L.ba_cuda_device_gpu.argtypes = [vp, C.c_int, i32p]
     L.ba_cuda_destroy.argtypes = [vp]
     L.ba_cuda_destroy.restype = None
     L.ba_cuda_last_error.restype = C.c_char_p
@@ -159,14 +163,29 @@ def device_to_host(ptr: int, nbytes: int) -> bytes:
 
 
 class Engine:
-    def __init__(self, cfg: abi.EngineCfg, lib_path: Optional[str] = None):
+    def __init__(self, cfg: abi.EngineCfg, lib_path: Optional[str] = None, gpus: Optional[Sequence[int]] = None,
+                 gpu_of_device: Optional[Sequence[int]] = None):
+        """One engine on cfg.cuda_device; with ``gpus`` (CUDA ordinals, repeats allowed) one engine over those GPUs
+        (ba_cuda_create_multi): devices are placed by ``gpu_of_device`` (indices into gpus) or, without it, with the
+        devices of a mixer kept together and groups dealt out round robin.  Every method works the same either way."""
         self.cfg = cfg
         self.L = load_library(lib_path)
         desc, self._keep = abi.build_desc(cfg)
         h = C.c_void_p()
-        rc = self.L.ba_cuda_create(C.byref(desc), C.byref(h))
+        if gpus is None:
+            if gpu_of_device is not None:
+                raise ValueError("gpu_of_device needs gpus")
+            rc = self.L.ba_cuda_create(C.byref(desc), C.byref(h))
+            where = "ba_cuda_create"
+        else:
+            if gpu_of_device is not None and len(gpu_of_device) != len(cfg.devices):
+                raise ValueError("gpu_of_device has %d entries for %d devices" % (len(gpu_of_device), len(cfg.devices)))
+            g = (C.c_int32 * max(1, len(gpus)))(*gpus)
+            m = None if gpu_of_device is None else (C.c_int32 * max(1, len(gpu_of_device)))(*gpu_of_device)
+            rc = self.L.ba_cuda_create_multi(C.byref(desc), g, len(gpus), m, C.byref(h))
+            where = "ba_cuda_create_multi"
         if rc != 0:
-            raise EngineError("ba_cuda_create", rc, self.L.ba_cuda_last_error().decode())
+            raise EngineError(where, rc, self.L.ba_cuda_last_error().decode())
         self.h = h
         self._pins: List[object] = []
 
@@ -277,6 +296,12 @@ class Engine:
         ms = C.c_float()
         self._check("ba_cuda_mark_ms", self.L.ba_cuda_mark_ms(self.h, a, b, C.byref(ms)))
         return ms.value
+
+    def device_gpu(self, dev: int) -> int:
+        """CUDA ordinal that device ``dev`` runs on: where its device-resident stream and device results must live."""
+        n = C.c_int32()
+        self._check("ba_cuda_device_gpu", self.L.ba_cuda_device_gpu(self.h, dev, C.byref(n)))
+        return n.value
 
     def launch_count(self) -> int:
         n = C.c_uint64()

@@ -188,7 +188,7 @@ typedef struct ba_step_out {
     const ba_channel_status* status; /* [batch][channel] */
     uint64_t frames_done;  /* FFT frames consumed from this device's stream so far */
     /* BA_FLAG_SKIP_SILENT_ROWS only (else NULL / 0): */
-    const float* rows;     /* [n_rows][wave_batch]: the rows of the whole step (all devices) that are not silence, packed */
+    const float* rows;     /* [n_rows][wave_batch]: the rows of the whole step (all devices of that GPU) that are not silence, packed */
     const int32_t* row_of; /* [channel][max_batches_per_step] for this device: index into rows, or -1 = wave_batch samples of +0.0f */
     uint32_t n_rows;
     int32_t row_of_stride; /* = max_batches_per_step */
@@ -229,6 +229,25 @@ typedef struct ba_engine ba_engine;
 /* Replaces init_demod()/gpu_fft_prepare (src/boondock_airband.cpp:253-266,316-332): builds the
  * window (.cpp:357-373), twiddles, per-channel constants and the resident per-channel state. */
 BA_API int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out);
+/*
+ * One engine over several GPUs: a group of ordinary engines ("members"), one per GPU that receives devices, behind one
+ * handle.  No data moves between GPUs: every device runs on exactly one of them, and a mixer's inputs stay together.
+ *   gpus[0..n_gpus)      CUDA ordinals; one may repeat (two members on one GPU).  desc->cuda_device is ignored.
+ *   gpu_of_device        NULL, or desc->device_count indices into gpus.  NULL places devices joined by a mixer (transitively)
+ *                        as one group, groups in the order of their first device, group k on gpus[k % n_gpus]; without
+ *                        mixers device i goes to gpus[i % n_gpus].  An explicit map may not split a mixer's inputs.
+ * A GPU that gets no device gets no member and is not touched.  BA_ERR_BAD_ARG for n_gpus < 1, an ordinal that is not
+ * visible, an index out of range or a split mixer.
+ * Every entry point below accepts the handle.  Device and mixer indices stay those of desc; per-device and per-mixer
+ * calls go to the member that holds the device or mixer.  ba_cuda_process() runs every member's pass, in member order,
+ * and returns their common ticket (members' tickets move in lockstep); ba_cuda_collect() waits for the member of the
+ * device only.  ticket_ms, copy_ms, kernel_ms and mark_ms give the maximum over members; step_bytes and launch_count the
+ * sum; ba_cuda_mark() records on every member.  After an error from any member the handle is only good for
+ * ba_cuda_destroy() (a failed ba_cuda_process() or CUDA error makes every later call return BA_ERR_STATE). */
+BA_API int ba_cuda_create_multi(const ba_engine_desc* desc, const int32_t* gpus, int32_t n_gpus, const int32_t* gpu_of_device, ba_engine** out);
+/* The CUDA ordinal device `dev` runs on (a plain engine: its cuda_device).  Memory given to ba_cuda_attach_device_stream()
+ * must be on that GPU, and the BA_FLAG_RESULTS_ON_DEVICE pointers of the device point there. */
+BA_API int ba_cuda_device_gpu(ba_engine* e, int dev, int32_t* cuda_ordinal);
 /* Replaces gpu_fft_release (src/boondock_airband.cpp:385-388). */
 BA_API void ba_cuda_destroy(ba_engine* e);
 /* Text of the most recent failure on this thread (never NULL). */
