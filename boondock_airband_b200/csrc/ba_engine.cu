@@ -78,6 +78,22 @@ int fail(int code, const char* fmt, ...) {
         }                                                                               \
     } while (0)
 #define FORWARD_DEV(e, dev, call) FORWARD(e, dev, dev_member, dev_local, "device", call)
+/* a per-channel call goes to the member that demodulates the channel, under its device and channel index there */
+#define FORWARD_CHAN(e, dev, channel, call)                                                              \
+    do {                                                                                                  \
+        if ((e) && !(e)->members.empty() && (dev) >= 0 && (dev) < (int)(e)->ch_member.size() &&           \
+            !(e)->ch_member[dev].empty() && !(e)->broken) {                                               \
+            ba_engine* g_ = (e);                                                                          \
+            if ((channel) < 0 || (channel) >= (int)g_->ch_member[dev].size())                             \
+                return fail(BA_ERR_BAD_ARG, "device %d has no channel %d", (int)(dev), (int)(channel));   \
+            e = g_->members[g_->ch_member[dev][channel]];                                                 \
+            const int d_ = g_->ch_dev[dev][channel];                                                      \
+            channel = g_->ch_local[dev][channel];                                                         \
+            dev = d_;                                                                                     \
+            return group_rc(g_, (call));                                                                  \
+        }                                                                                                 \
+        FORWARD_DEV(e, dev, call);                                                                        \
+    } while (0)
 #define FORWARD_MIXER(e, mixer, call) FORWARD(e, mixer, mix_member, mix_local, "mixer", call)
 
 uint32_t pow2_at_least(uint64_t v) {
@@ -121,6 +137,8 @@ struct Dev {
     size_t attached_cap = 0, attached_valid = 0;
     uint64_t frames_done = 0, batches_done = 0;
     bool injected = false;
+    bool shadow = false; /* a follower's copy of a split input (ba_cuda_create_multi_split): no input of its own, its picks are
+                            shipped from the home, its plan is the home's; a member's shadows come after its own devices */
     /* picks, bins */
     float2* d_picks = nullptr;
     float* d_mags = nullptr;
@@ -192,6 +210,38 @@ struct Slot {
     std::vector<int> n_batches; /* per device */
     std::vector<uint64_t> frames_done;
     uint64_t h2d_bytes = 0, d2h_bytes = 0;
+    /* channel sharding: the ship and gather job tables of this ticket, and the events behind the two launches */
+    unsigned char* d_xfer = nullptr;
+    unsigned char* h_xfer = nullptr;
+    cudaEvent_t ev_ship = nullptr, ev_gather = nullptr;
+};
+
+/* a host->device piece of input bytes */
+struct Piece {
+    unsigned char* dst;
+    const unsigned char* src;
+    size_t n;
+};
+
+/* channel sharding (ba_cuda_create_multi_split), as a member sees it */
+struct ShipTo { /* on a home: one follower of one of its inputs */
+    int dev = 0;                /* the input, index in this member */
+    ba_engine* to = nullptr;    /* the follower */
+    int shadow = 0;             /* the follower's shadow of the input */
+    std::vector<int> home_ch;   /* per channel of the shadow: the channel here */
+    std::vector<char> picks;    /* and whether its picked IQ travels with the magnitudes */
+};
+struct GatherTo { /* on a follower: one of its shadows */
+    int shadow = 0;
+    ba_engine* home = nullptr;
+    int dev = 0;                /* the input, index in the home */
+    std::vector<int> home_ch;
+};
+
+/* what ba_cuda_create_multi_split() asks of one member beyond its descriptor */
+struct CreateOpts {
+    int n_shadow = 0;                       /* the last n_shadow devices of the descriptor are shadows */
+    std::vector<std::vector<char>> remote;  /* per own device: per channel, demodulated on another member (may be empty) */
 };
 
 /* ring bytes a ticket queued for copying: given back to the producers (bufs) once `ev` has fired */
@@ -257,7 +307,30 @@ struct ba_engine {
     std::vector<ba_engine*> members;
     std::vector<int> dev_member, dev_local; /* per device of the group's descriptor */
     std::vector<int> mix_member, mix_local; /* per mixer */
+    std::vector<std::vector<int>> ch_member, ch_dev, ch_local; /* per device: per channel, member / device / channel that runs it
+                                                                  (empty: the device is not split) */
     bool broken = false;                    /* a member failed in a way that may leave the members out of step */
+    /* a member of a group that splits channels */
+    int n_own = 0;        /* devices that are not shadows (the first n_own) */
+    int own_channels = 0; /* their channels */
+    int n_launch = 0;     /* channels in the demodulator's launch order (those of a split input that run elsewhere are left out) */
+    std::vector<ShipTo> ship;
+    std::vector<GatherTo> gather;
+    size_t xfer_gather_off = 0; /* where the gather table starts in a slot's h_xfer / d_xfer */
+    /* one pass of ba_cuda_process(), carried from one stage to the next */
+    struct {
+        int ticket = -1;
+        std::vector<Piece> pieces;
+        int n_carry = 0;
+        bool any_ring = false;
+        int phases = 1;
+        std::vector<int> k1_count, k1_tiles, k2_any, k1_plain, k1_plain_tiles;
+        int mix_max_emit = 0, mix_max_stash = 0;
+        ba::K3InDyn* d_in_dyn = nullptr;
+        ba::K3MixDyn* d_mix_dyn = nullptr;
+        int n_ship = 0, n_gather = 0;
+        uint32_t ship_frames = 0, gather_samples = 0;
+    } pass;
 };
 
 namespace {
@@ -347,6 +420,13 @@ void free_engine(ba_engine* e) {
             cudaEventDestroy(s.ev_out0);
         for (cudaEvent_t ev : s.ev_k)
             cudaEventDestroy(ev);
+        cudaFree(s.d_xfer);
+        if (s.h_xfer)
+            cudaFreeHost(s.h_xfer);
+        if (s.ev_ship)
+            cudaEventDestroy(s.ev_ship);
+        if (s.ev_gather)
+            cudaEventDestroy(s.ev_gather);
     }
     for (cudaEvent_t ev : e->marks)
         if (ev)
@@ -605,7 +685,13 @@ void ba_cuda_destroy(ba_engine* e) {
     free_engine(e);
 }
 
+static int create_engine(const ba_engine_desc* desc, const CreateOpts* opts, ba_engine** out);
+
 int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
+    return create_engine(desc, nullptr, out);
+}
+
+static int create_engine(const ba_engine_desc* desc, const CreateOpts* opts, ba_engine** out) {
     using namespace ba;
     if (!desc || !out)
         return fail(BA_ERR_BAD_ARG, "null argument");
@@ -697,6 +783,7 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
         if (!d)
             return fail(BA_ERR_NOMEM, "host allocation");
         e->dev.push_back(d);
+        d->shadow = opts && di >= desc->device_count - opts->n_shadow;
         d->cfg = dd;
         d->chans.assign(dd.channels, dd.channels + dd.channel_count);
         d->cfg.channels = nullptr;
@@ -718,6 +805,10 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
         d->frame_bytes = d->sample_bytes * (size_t)N;
         d->first_chan = e->total_channels;
         e->total_channels += d->C;
+        if (!d->shadow) {
+            e->n_own++;
+            e->own_channels += d->C;
+        }
         e->max_channels = std::max(e->max_channels, d->C);
         for (size_t ci = 0; ci < d->chans.size(); ci++) {
             const ba_channel_desc& c = d->chans[ci];
@@ -734,19 +825,21 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
         }
         e->any_afc |= d->any_afc;
         e->any_iq |= d->any_iq;
-        /* host ring, config.cpp:796-805 */
+        /* host ring, config.cpp:796-805 (a shadow has no input: no ring, no stream window) */
         d->buf_size = model::ring_bytes(ring_min, dd.bytes_per_sample, dd.sample_rate, e->wave_rate);
         d->mirror = d->frame_bytes;
-        if (cudaHostAlloc((void**)&d->ring, d->buf_size + d->mirror, cudaHostAllocDefault) != cudaSuccess)
-            return fail(BA_ERR_NOMEM, "pinned ring of %zu bytes", d->buf_size + d->mirror);
-        memset(d->ring, 0, d->buf_size + d->mirror);
+        if (!d->shadow) {
+            if (cudaHostAlloc((void**)&d->ring, d->buf_size + d->mirror, cudaHostAllocDefault) != cudaSuccess)
+                return fail(BA_ERR_NOMEM, "pinned ring of %zu bytes", d->buf_size + d->mirror);
+            memset(d->ring, 0, d->buf_size + d->mirror);
+        }
         /* HBM: stream window (two halves), pick ring, bins */
-        d->d_cap = (size_t)(frames_cap + 2) * d->hop_bytes + 2 * d->frame_bytes + 64;
+        d->d_cap = d->shadow ? 0 : (size_t)(frames_cap + 2) * d->hop_bytes + 2 * d->frame_bytes + 64;
         /* two tickets may be in flight on the pick ring: the demodulator of one reads behind the channelizer of the next */
         d->ring_len = pow2_at_least((uint64_t)(2 * e->max_batches + 1) * e->B + 2 * BA_E);
         /* picked-bin IQ is kept only where a demodulator reads it (or a test asked for it); magnitudes always */
         const bool keep_picks = d->any_raw || (e->flags & BA_FLAG_KEEP_PICKS);
-        if (cudaMalloc((void**)&d->d_buf[0], d->d_cap) != cudaSuccess || cudaMalloc((void**)&d->d_buf[1], d->d_cap) != cudaSuccess ||
+        if ((!d->shadow && (cudaMalloc((void**)&d->d_buf[0], d->d_cap) != cudaSuccess || cudaMalloc((void**)&d->d_buf[1], d->d_cap) != cudaSuccess)) ||
             (keep_picks && cudaMalloc((void**)&d->d_picks, sizeof(float2) * (size_t)d->ring_len * d->C) != cudaSuccess) ||
             cudaMalloc((void**)&d->d_mags, sizeof(float) * (size_t)d->ring_len * d->C) != cudaSuccess ||
             cudaMalloc((void**)&d->d_bins, sizeof(uint32_t) * d->c_pad) != cudaSuccess)
@@ -814,11 +907,17 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
         CU(cudaMemcpy(d.d_bins, bins.data(), sizeof(uint32_t) * d.c_pad, cudaMemcpyHostToDevice));
     }
     /* launch order: group channels of one kind together (plain AM, other AM, filtered/NFM, CTCSS) so that the lanes of a warp
-     * run the same code; plain AM channels come first and go to their own kernel */
+     * run the same code; plain AM channels come first and go to their own kernel.  Channels of a split input that another
+     * member demodulates are left out. */
     {
-        std::vector<int32_t> order(TC);
-        for (int i = 0; i < TC; i++)
-            order[i] = i;
+        std::vector<int32_t> order;
+        for (int i = 0; i < TC; i++) {
+            const K2Chan& k = e->h_chan[i];
+            if (opts && k.dev < (int)opts->remote.size() && !opts->remote[k.dev].empty() && opts->remote[k.dev][k.col])
+                continue;
+            order.push_back(i);
+        }
+        e->n_launch = (int)order.size();
         auto plain = [&](int i) {
             const K2Chan& k = e->h_chan[i];
             const Dev& dv = *e->dev[k.dev];
@@ -832,9 +931,10 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
         };
         std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return kind(a) < kind(b); });
         e->n_plain = 0;
-        for (int i = 0; i < TC; i++)
+        for (int32_t i : order)
             e->n_plain += plain(i) ? 1 : 0;
-        CU(cudaMemcpy(e->d_order, order.data(), sizeof(int32_t) * TC, cudaMemcpyHostToDevice));
+        if (!order.empty())
+            CU(cudaMemcpy(e->d_order, order.data(), sizeof(int32_t) * order.size(), cudaMemcpyHostToDevice));
     }
     CU(cudaMemcpy(e->d_chan, e->h_chan.data(), sizeof(K2Chan) * TC, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(e->d_state, h_state.data(), sizeof(K2State) * TC, cudaMemcpyHostToDevice));
@@ -979,7 +1079,7 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
     {
         const uint64_t frames_per_step = (uint64_t)e->dev.size() * e->max_batches * e->B;
         const bool big_step = frames_per_step / (uint64_t)std::max(1, e->tile_frames) >= 16ull * e->sm_count * e->k1_ctas_per_sm;
-        if (e->n_plain == e->total_channels && big_step && !(e->flags & BA_FLAG_RESULTS_ON_DEVICE)) /* with no copy waiting for K2, beside K1 is the shorter schedule */
+        if (e->n_plain == e->n_launch && big_step && !(e->flags & BA_FLAG_RESULTS_ON_DEVICE)) /* with no copy waiting for K2, beside K1 is the shorter schedule */
             e->serial_k2 = true;
         if (const char* v = getenv("BA_CUDA_SERIAL_K2")) /* tuning runs only: 0 / 1 overrides the rule (AFC always serialises) */
             e->serial_k2 = e->any_afc || atoi(v) != 0;
@@ -991,6 +1091,11 @@ int ba_cuda_create(const ba_engine_desc* desc, ba_engine** out) {
 }
 
 int ba_cuda_create_multi(const ba_engine_desc* desc, const int32_t* gpus, int32_t n_gpus, const int32_t* gpu_of_device, ba_engine** out) {
+    return ba_cuda_create_multi_split(desc, gpus, n_gpus, gpu_of_device, nullptr, out);
+}
+
+int ba_cuda_create_multi_split(const ba_engine_desc* desc, const int32_t* gpus, int32_t n_gpus, const int32_t* gpu_of_device,
+                               const int32_t* const* gpu_of_channel, ba_engine** out) {
     if (!desc || !out || !gpus)
         return fail(BA_ERR_BAD_ARG, "null argument");
     *out = nullptr;
@@ -1059,22 +1164,109 @@ int ba_cuda_create_multi(const ba_engine_desc* desc, const int32_t* gpus, int32_
         }
     }
 
+    /* channels: ch_where[d] = per channel an index into gpus, or empty when the whole device stays at its home */
+    std::vector<std::vector<int>> ch_where(nd);
+    if (gpu_of_channel) {
+        for (int d = 0; d < nd; d++) {
+            const int32_t* map = gpu_of_channel[d];
+            const ba_device_desc& dd = desc->devices[d];
+            if (!map)
+                continue;
+            if (dd.channel_count <= 0 || !dd.channels)
+                return fail(BA_ERR_BAD_ARG, "device %d has no channels", d);
+            bool split = false;
+            for (int c = 0; c < dd.channel_count; c++) {
+                if (map[c] < 0 || map[c] >= n_gpus)
+                    return fail(BA_ERR_BAD_ARG, "gpu_of_channel[%d][%d] = %d is not an index into the %d gpus", d, c, map[c], n_gpus);
+                split = split || map[c] != where[d];
+            }
+            if (!split)
+                continue;
+            for (int c = 0; c < dd.channel_count; c++)
+                if (dd.channels[c].afc & 0xff)
+                    return fail(BA_ERR_BAD_ARG, "device %d cannot be split: channel %d has AFC, which moves its bins on the home's channelizer every batch", d, c);
+            for (int c = 0; c < dd.channel_count; c++) {
+                const int a = gpus[where[d]], b = gpus[map[c]];
+                if (a == b)
+                    continue;
+                int ab = 0, ba_ = 0;
+                if (cudaDeviceCanAccessPeer(&ab, a, b) != cudaSuccess || cudaDeviceCanAccessPeer(&ba_, b, a) != cudaSuccess || !ab || !ba_)
+                    return fail(BA_ERR_BAD_ARG, "device %d channel %d: GPU %d and its home GPU %d have no peer access to each other", d, c, b, a);
+            }
+            ch_where[d].assign(map, map + dd.channel_count);
+        }
+    }
+    /* peer access both ways between the home and every other GPU of a split device (already enabled is fine) */
+    for (int d = 0; d < nd; d++)
+        for (size_t c = 0; c < ch_where[d].size(); c++) {
+            const int a = gpus[where[d]], b = gpus[ch_where[d][c]];
+            if (a == b)
+                continue;
+            for (int k = 0; k < 2; k++) {
+                if (cudaSetDevice(k ? b : a) != cudaSuccess)
+                    return fail(BA_ERR_CUDA, "cudaSetDevice(%d) failed", k ? b : a);
+                const cudaError_t pe = cudaDeviceEnablePeerAccess(k ? a : b, 0);
+                if (pe == cudaErrorPeerAccessAlreadyEnabled)
+                    cudaGetLastError();
+                else if (pe != cudaSuccess)
+                    return fail(BA_ERR_CUDA, "peer access from GPU %d to GPU %d: %s", k ? b : a, k ? a : b, cudaGetErrorString(pe));
+            }
+        }
+
     ba_engine* g = new (std::nothrow) ba_engine();
     if (!g)
         return fail(BA_ERR_NOMEM, "host allocation");
+    auto give_up = [&](int rc) {
+        for (ba_engine* x : g->members)
+            free_engine(x);
+        delete g;
+        return rc;
+    };
     g->dev_member.assign(nd, -1);
     g->dev_local.assign(nd, -1);
     g->mix_member.assign(n_mixers, -1);
     g->mix_local.assign(n_mixers, -1);
-    /* one member per entry of gpus that received devices, in the order of gpus; a mixer without inputs goes with device 0 */
+    g->ch_member.resize(nd);
+    g->ch_dev.resize(nd);
+    g->ch_local.resize(nd);
+    /* shadow_of[d][k]: index of gpus[k]'s shadow of split device d in its member, -1 if none */
+    std::vector<std::vector<int>> shadow_of(nd, std::vector<int>(n_gpus, -1));
+    std::vector<int> member_of(n_gpus, -1);
+    /* one member per entry of gpus that received devices or channels, in the order of gpus; its own devices first, then its
+     * shadows; a mixer without inputs goes with device 0 */
     for (int k = 0; k < n_gpus; k++) {
         std::vector<ba_device_desc> devs;
+        CreateOpts opts;
         for (int d = 0; d < nd; d++)
             if (where[d] == k) {
                 g->dev_member[d] = (int)g->members.size();
                 g->dev_local[d] = (int)devs.size();
                 devs.push_back(desc->devices[d]);
+                std::vector<char> remote;
+                for (int w : ch_where[d])
+                    remote.push_back(w != k);
+                opts.remote.push_back(remote);
             }
+        std::vector<std::vector<ba_channel_desc>> shard_chans;
+        for (int d = 0; d < nd; d++) {
+            if (where[d] == k || ch_where[d].empty())
+                continue;
+            std::vector<ba_channel_desc> sc;
+            for (size_t c = 0; c < ch_where[d].size(); c++)
+                if (ch_where[d][c] == k)
+                    sc.push_back(desc->devices[d].channels[c]);
+            if (sc.empty())
+                continue;
+            shadow_of[d][k] = (int)devs.size();
+            devs.push_back(desc->devices[d]);
+            shard_chans.push_back(sc);
+            opts.n_shadow++;
+        }
+        for (int i = 0; i < opts.n_shadow; i++) {
+            ba_device_desc& sd = devs[devs.size() - opts.n_shadow + i];
+            sd.channels = shard_chans[i].data();
+            sd.channel_count = (int32_t)shard_chans[i].size();
+        }
         if (devs.empty())
             continue;
         std::vector<ba_mixer_desc> mixers;
@@ -1099,14 +1291,73 @@ int ba_cuda_create_multi(const ba_engine_desc* desc, const int32_t* gpus, int32_
         sub.mixer_count = (int32_t)mixers.size();
         sub.mixers = mixers.empty() ? nullptr : mixers.data();
         ba_engine* m = nullptr;
-        const int rc = ba_cuda_create(&sub, &m);
-        if (rc != BA_OK) {
-            for (ba_engine* x : g->members)
-                free_engine(x);
-            delete g;
-            return rc;
-        }
+        const int rc = create_engine(&sub, &opts, &m);
+        if (rc != BA_OK)
+            return give_up(rc);
+        member_of[k] = (int)g->members.size();
         g->members.push_back(m);
+    }
+    /* who runs each channel of a split device; the ship and gather links between its home and its followers */
+    for (int d = 0; d < nd; d++) {
+        if (ch_where[d].empty())
+            continue;
+        ba_engine* home = g->members[g->dev_member[d]];
+        std::vector<int> next(n_gpus, 0);
+        for (size_t c = 0; c < ch_where[d].size(); c++) {
+            const int k = ch_where[d][c];
+            if (k == where[d]) {
+                g->ch_member[d].push_back(g->dev_member[d]);
+                g->ch_dev[d].push_back(g->dev_local[d]);
+                g->ch_local[d].push_back((int)c);
+            } else {
+                g->ch_member[d].push_back(member_of[k]);
+                g->ch_dev[d].push_back(shadow_of[d][k]);
+                g->ch_local[d].push_back(next[k]++);
+            }
+        }
+        for (int k = 0; k < n_gpus; k++) {
+            if (shadow_of[d][k] < 0)
+                continue;
+            ba_engine* f = g->members[member_of[k]];
+            ShipTo st;
+            st.dev = g->dev_local[d];
+            st.to = f;
+            st.shadow = shadow_of[d][k];
+            GatherTo gt;
+            gt.shadow = shadow_of[d][k];
+            gt.home = home;
+            gt.dev = g->dev_local[d];
+            const Dev& sd = *f->dev[gt.shadow];
+            for (size_t c = 0; c < ch_where[d].size(); c++)
+                if (ch_where[d][c] == k) {
+                    const int lc = (int)st.home_ch.size();
+                    st.home_ch.push_back((int)c);
+                    st.picks.push_back(f->h_chan[sd.first_chan + lc].needs_raw_iq || (desc->flags & BA_FLAG_KEEP_PICKS));
+                }
+            gt.home_ch = st.home_ch;
+            home->ship.push_back(st);
+            f->gather.push_back(gt);
+        }
+    }
+    /* every member that ships or gathers: per slot a job table and the two events */
+    for (ba_engine* m : g->members) {
+        if (m->ship.empty() && m->gather.empty())
+            continue;
+        if (cudaSetDevice(m->cuda_device) != cudaSuccess)
+            return give_up(fail(BA_ERR_CUDA, "cudaSetDevice(%d) failed", m->cuda_device));
+        size_t n_ship = 0, n_gather = 0;
+        for (const ShipTo& st : m->ship)
+            n_ship += st.home_ch.size();
+        for (const GatherTo& gt : m->gather)
+            n_gather += gt.home_ch.size();
+        m->xfer_gather_off = (sizeof(ba::XShip) * n_ship + 15) & ~(size_t)15;
+        const size_t bytes = std::max<size_t>(16, m->xfer_gather_off + sizeof(ba::XGather) * n_gather);
+        for (Slot& s : m->slot) {
+            if (cudaMalloc((void**)&s.d_xfer, bytes) != cudaSuccess || cudaHostAlloc((void**)&s.h_xfer, bytes, cudaHostAllocDefault) != cudaSuccess)
+                return give_up(fail(BA_ERR_NOMEM, "ship/gather tables"));
+            if (cudaEventCreateWithFlags(&s.ev_ship, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&s.ev_gather, cudaEventDisableTiming) != cudaSuccess)
+                return give_up(fail(BA_ERR_CUDA, "ship/gather events"));
+        }
     }
     *out = g;
     return BA_OK;
@@ -1118,6 +1369,18 @@ int ba_cuda_device_gpu(ba_engine* e, int dev, int32_t* cuda_ordinal) {
     FORWARD_DEV(e, dev, ba_cuda_device_gpu(e, dev, cuda_ordinal));
     if (!e || dev < 0 || dev >= (int)e->dev.size())
         return fail(BA_ERR_BAD_ARG, "bad engine or device index %d", dev);
+    *cuda_ordinal = e->cuda_device;
+    return BA_OK;
+}
+
+int ba_cuda_channel_gpu(ba_engine* e, int dev, int channel, int32_t* cuda_ordinal) {
+    if (!cuda_ordinal)
+        return fail(BA_ERR_BAD_ARG, "null argument");
+    FORWARD_CHAN(e, dev, channel, ba_cuda_channel_gpu(e, dev, channel, cuda_ordinal));
+    if (!e || dev < 0 || dev >= (int)e->dev.size())
+        return fail(BA_ERR_BAD_ARG, "bad engine or device index %d", dev);
+    if (channel < 0 || channel >= e->dev[dev]->C)
+        return fail(BA_ERR_BAD_ARG, "device %d has no channel %d", dev, channel);
     *cuda_ordinal = e->cuda_device;
     return BA_OK;
 }
@@ -1320,25 +1583,16 @@ static uint64_t frame_room(const ba_engine* e, const Dev& d) {
     return limit > d.frames_done ? limit - d.frames_done : 0;
 }
 
-int ba_cuda_process(ba_engine* e) {
-    if (e && !e->members.empty()) { /* every member's pass; their tickets move in lockstep */
-        int ticket = -1;
-        const int rc = each_member(e, [&](ba_engine* m) {
-            const int t = ba_cuda_process(m);
-            if (t >= 0 && ticket >= 0 && t != ticket)
-                return fail(BA_ERR_STATE, "member tickets %d and %d differ", ticket, t);
-            ticket = t;
-            return t;
-        });
-        if (rc < 0)
-            e->broken = true;
-        return rc < 0 ? rc : ticket;
-    }
+/* ba_cuda_process() in four stages: 1 plan, 2 input copies + K1 + ship, 3 K2 + gather, 4 K3 + pack + device->host copies.  A
+ * plain engine runs them back to back; a group runs each stage on every member before the next stage, so that the events
+ * one member waits for (a home's ship, a follower's gather) have been recorded by then whichever way round the two are. */
+
+/* 1: which slot, what to wait for, and how many frames and batches every input runs (host work only) */
+static int stage_plan(ba_engine* e) {
     using namespace ba;
-    if (!e)
-        return fail(BA_ERR_BAD_ARG, "null engine");
     USE_DEVICE(e);
     const int ticket = e->next_ticket;
+    e->pass.ticket = ticket;
     Slot& s = e->slot[ticket % BA_SLOTS];
     release_rings(e, false);
     while (ring_release_pending(e, s.ev_ring)) /* this slot's previous ticket (three steps back) still holds ring bytes: its copies finished long ago */
@@ -1369,18 +1623,18 @@ int ba_cuda_process(ba_engine* e) {
     /* 1. move new bytes to HBM and decide how many frames and batches every input runs */
     std::vector<size_t>& ring_taken = s.ring_taken;
     std::fill(ring_taken.begin(), ring_taken.end(), (size_t)0);
-    bool any_ring = false;
+    bool& any_ring = e->pass.any_ring;
+    any_ring = false;
     /* host->device pieces are queued behind ALL the device->device carries of the step, so that the copy engine runs the
      * big transfers back to back instead of alternating directions per input */
-    struct Piece {
-        unsigned char* dst;
-        const unsigned char* src;
-        size_t n;
-    };
-    std::vector<Piece> pieces;
-    int n_carry = 0;
+    std::vector<Piece>& pieces = e->pass.pieces;
+    pieces.clear();
+    int& n_carry = e->pass.n_carry;
+    n_carry = 0;
     for (size_t di = 0; di < nd; di++) {
         Dev& d = *e->dev[di];
+        if (d.shadow) /* planned by its home (copy_shadow_plans) */
+            continue;
         const uint64_t room = frame_room(e, d);
         uint64_t total = 0;
         if (d.injected) {
@@ -1456,6 +1710,92 @@ int ba_cuda_process(ba_engine* e) {
         d.step_batch0 = d.batches_done;
         d.step_batches = (int)nb;
     }
+    return ticket;
+}
+
+/* K1 of phase ph (the launch descriptors are in the slot) */
+static int launch_k1(ba_engine* e, Slot& s, int ph) {
+    using namespace ba;
+    const size_t nd = e->dev.size();
+    const std::vector<int>&k1_count = e->pass.k1_count, &k1_tiles = e->pass.k1_tiles, &k1_plain = e->pass.k1_plain, &k1_plain_tiles = e->pass.k1_plain_tiles;
+    K1Device* d_k1 = reinterpret_cast<K1Device*>(s.d_desc);
+    {
+        CU(cudaEventRecord(s.ev_k[4 * ph + 0], e->s_k));
+        /* Inputs without AFC never run the instantiation that also writes the spectrum: the two are compiled apart and may
+         * round the FFT differently in the last bit, and an input's audio must not depend on whether another input of its
+         * engine has AFC (nor on which member of a multi-GPU group it was placed in). */
+        for (int afc = 0; afc < 2; afc++) {
+            const int first = afc ? k1_plain[ph] : 0;
+            const int n_dev = afc ? k1_count[ph] - k1_plain[ph] : k1_plain[ph];
+            if (n_dev == 0)
+                continue;
+            K1Params p;
+            p.dev = d_k1 + (size_t)ph * nd + first;
+            p.n_dev = n_dev;
+            p.tile_frames = e->tile_frames;
+            p.n_tiles = afc ? k1_tiles[ph] - k1_plain_tiles[ph] : k1_plain_tiles[ph];
+            p.window = e->d_window;
+            p.twiddle = e->d_twiddle;
+            p.raw_bytes = e->raw_bytes;
+            p.max_channels = e->max_channels;
+            p.tile_counter = e->d_tile_counter;
+            const int ctas = std::min(p.n_tiles, e->sm_count * e->k1_ctas_per_sm);
+            CU(cudaMemsetAsync(e->d_tile_counter, 0, sizeof(uint32_t), e->s_k));
+            int rc = k1_launch(e->fft_size, p, ctas, afc != 0, e->s_k);
+            if (rc != 0)
+                return fail(BA_ERR_CUDA, "channelize launch: %s", cudaGetErrorString((cudaError_t)rc));
+            e->launches++;
+        }
+        CU(cudaEventRecord(s.ev_k[4 * ph + 1], e->s_k));
+        CU(cudaEventRecord(s.ev_k1, e->s_k));
+    }
+    return BA_OK;
+}
+
+/* K2 of phase ph */
+static int launch_k2(ba_engine* e, Slot& s, int ph) {
+    using namespace ba;
+    const size_t nd = e->dev.size();
+    const int B = e->B;
+    cudaStream_t k2s = e->serial_k2 ? e->s_k : e->s_k2;
+    K2Dyn* d_dyn = reinterpret_cast<K2Dyn*>(s.d_desc + (size_t)e->max_phases * nd * sizeof(K1Device));
+    {
+        if (k2s != e->s_k)
+            CU(cudaStreamWaitEvent(k2s, s.ev_k1, 0));
+        if (ph == 0) /* a shadow's picks have arrived */
+            for (const GatherTo& gt : e->gather)
+                CU(cudaStreamWaitEvent(k2s, gt.home->slot[e->pass.ticket % BA_SLOTS].ev_ship, 0));
+        CU(cudaEventRecord(s.ev_k[4 * ph + 2], k2s));
+        if (e->pass.k2_any[ph]) {
+            K2Params p;
+            p.chan = e->d_chan;
+            p.state = e->d_state;
+            p.dyn = d_dyn + (size_t)ph * nd;
+            p.order = e->d_order;
+            p.n_channels = e->n_launch;
+            p.wave_batch = B;
+            p.sincos = e->d_sincos;
+            int rc = k2_launch(p, e->n_plain, e->sm_count, k2s, e->s_k2b, e->ev_fork, e->ev_join);
+            if (rc != 0)
+                return fail(BA_ERR_CUDA, "demod launch: %s", cudaGetErrorString((cudaError_t)rc));
+            e->launches += (e->n_plain > 0 ? 1 : 0) + (e->n_launch > e->n_plain ? 1 : 0);
+        }
+        CU(cudaEventRecord(s.ev_k[4 * ph + 3], k2s));
+    }
+    return BA_OK;
+}
+
+/* 2: input bytes to HBM, descriptors, K1 of the first phase, ship */
+static int stage_k1(ba_engine* e) {
+    using namespace ba;
+    USE_DEVICE(e);
+    const int ticket = e->pass.ticket;
+    Slot& s = e->slot[ticket % BA_SLOTS];
+    const size_t nd = e->dev.size();
+    const int B = e->B;
+    const std::vector<Piece>& pieces = e->pass.pieces;
+    std::vector<size_t>& ring_taken = s.ring_taken;
+    const int n_carry = e->pass.n_carry;
     if (n_carry) {
         /* one launch moves every input's tail; the list is read from pinned host memory in place */
         int rc = k1_carry_launch(s.h_carry, n_carry, e->s_in);
@@ -1475,7 +1815,7 @@ int ba_cuda_process(ba_engine* e) {
             CU(cudaStreamWaitEvent(e->s_in, s.ev_in2, 0));
         }
     }
-    if (any_ring) {
+    if (e->pass.any_ring) {
         /* the pinned rings are read by the copy engine: the bytes go back to the producers (bufs, .cpp:735) once this event has
          * fired - checked without blocking by release_rings() at the next call of any entry point, so that this thread can go
          * on planning and a producer thread can go on filling the ring while the copies and the kernels run */
@@ -1485,7 +1825,8 @@ int ba_cuda_process(ba_engine* e) {
     }
 
     /* 2. phases: one for ordinary inputs; an AFC input alternates K1/K2 per batch */
-    int phases = 1;
+    int& phases = e->pass.phases;
+    phases = 1;
     for (Dev* d : e->dev)
         if (d->any_afc)
             phases = std::max(phases, d->step_batches + 1);
@@ -1495,7 +1836,10 @@ int ba_cuda_process(ba_engine* e) {
     K2Dyn* d_dyn = reinterpret_cast<K2Dyn*>(s.d_desc + (size_t)e->max_phases * nd * sizeof(K1Device));
     /* K1 entries of a phase: inputs without AFC first, then the AFC inputs, which need the instantiation that also writes the
      * spectrum (k1_plain / k1_plain_tiles: entries and tiles of the first kind); each kind is one launch */
-    std::vector<int> k1_count(phases, 0), k1_tiles(phases, 0), k2_any(phases, 0), k1_plain(phases, 0), k1_plain_tiles(phases, 0);
+    std::vector<int>&k1_count = e->pass.k1_count, &k1_tiles = e->pass.k1_tiles, &k2_any = e->pass.k2_any, &k1_plain = e->pass.k1_plain,
+                    &k1_plain_tiles = e->pass.k1_plain_tiles;
+    for (std::vector<int>* v : {&k1_count, &k1_tiles, &k2_any, &k1_plain, &k1_plain_tiles})
+        v->assign(phases, 0);
     std::vector<size_t> order;
     for (int afc = 0; afc < 2; afc++)
         for (size_t di = 0; di < nd; di++)
@@ -1527,7 +1871,7 @@ int ba_cuda_process(ba_engine* e) {
                     f_end = f_begin;
                 b_first = ph;
             }
-            if (f_end > f_begin) {
+            if (f_end > f_begin && !d.shadow) { /* a shadow's picks come from its home */
                 K1Device& k = h_k1[(size_t)ph * nd + k1_count[ph]];
                 memset(&k, 0, sizeof(k));
                 const uint64_t off = f_begin * d.hop_bytes;
@@ -1571,9 +1915,13 @@ int ba_cuda_process(ba_engine* e) {
     }
     /* 2b. mixers: batch k of a mixer is mixed once every unmasked input has delivered its batch k; what an input
      * delivers beyond that is parked in the mixer FIFO */
-    int mix_max_emit = 0, mix_max_stash = 0;
-    K3InDyn* d_in_dyn = nullptr;
-    K3MixDyn* d_mix_dyn = nullptr;
+    int& mix_max_emit = e->pass.mix_max_emit;
+    int& mix_max_stash = e->pass.mix_max_stash;
+    K3InDyn*& d_in_dyn = e->pass.d_in_dyn;
+    K3MixDyn*& d_mix_dyn = e->pass.d_mix_dyn;
+    mix_max_emit = mix_max_stash = 0;
+    d_in_dyn = nullptr;
+    d_mix_dyn = nullptr;
     if (!e->mixers.empty()) {
         const size_t ni = std::max<size_t>(1, e->mix_in.size());
         K3InDyn* h_in_dyn = reinterpret_cast<K3InDyn*>(s.h_desc + e->mix_desc_off);
@@ -1620,70 +1968,138 @@ int ba_cuda_process(ba_engine* e) {
             mx.emitted = emit_end;
         }
     }
+    /* 2c. channel sharding: ship and gather jobs of this ticket */
+    if (!e->ship.empty() || !e->gather.empty()) {
+        XShip* h_ship = reinterpret_cast<XShip*>(s.h_xfer);
+        XGather* h_gather = reinterpret_cast<XGather*>(s.h_xfer + e->xfer_gather_off);
+        int& n_ship = e->pass.n_ship;
+        int& n_gather = e->pass.n_gather;
+        n_ship = n_gather = 0;
+        e->pass.ship_frames = e->pass.gather_samples = 0;
+        for (const ShipTo& st : e->ship) {
+            const Dev& d = *e->dev[st.dev];
+            const Dev& sd = *st.to->dev[st.shadow];
+            if (d.step_frames <= 0)
+                continue;
+            for (size_t k = 0; k < st.home_ch.size(); k++) {
+                XShip& j = h_ship[n_ship++];
+                const size_t hc = (size_t)st.home_ch[k];
+                j.src_mags = d.d_mags + hc * d.ring_len;
+                j.dst_mags = sd.d_mags + k * sd.ring_len;
+                j.src_picks = st.picks[k] ? d.d_picks + hc * d.ring_len : nullptr;
+                j.dst_picks = st.picks[k] ? sd.d_picks + k * sd.ring_len : nullptr;
+                j.frame0 = d.step_frame0;
+                j.n_frames = (uint32_t)d.step_frames;
+                j.ring_mask = d.ring_len - 1;
+            }
+            e->pass.ship_frames = std::max(e->pass.ship_frames, (uint32_t)d.step_frames);
+        }
+        for (const GatherTo& gt : e->gather) {
+            const Dev& sd = *e->dev[gt.shadow];
+            const Dev& hd = *gt.home->dev[gt.dev];
+            const Slot& hs = gt.home->slot[ticket % BA_SLOTS];
+            if (sd.step_batches <= 0)
+                continue;
+            for (size_t k = 0; k < gt.home_ch.size(); k++) {
+                XGather& j = h_gather[n_gather++];
+                const size_t hc = (size_t)gt.home_ch[k];
+                const size_t src = sd.wave_off + k * e->stride, dst = hd.wave_off + hc * e->stride;
+                j.src_wave = s.d_wave + src;
+                j.dst_wave = hs.d_wave + dst;
+                j.src_trace = s.d_trace ? s.d_trace + src : nullptr;
+                j.dst_trace = s.d_trace ? hs.d_trace + dst : nullptr;
+                const bool iq = sd.chans[k].has_iq_outputs != 0;
+                j.src_iq = iq ? s.d_iq + sd.iq_off + k * e->stride : nullptr;
+                j.dst_iq = iq ? hs.d_iq + hd.iq_off + hc * e->stride : nullptr;
+                j.src_status = s.d_status + sd.status_off + k;
+                j.dst_status = hs.d_status + hd.status_off + hc;
+                j.n_samples = (uint32_t)sd.step_batches * B;
+                j.n_batches = (uint32_t)sd.step_batches;
+                j.src_status_stride = (uint32_t)sd.C;
+                j.dst_status_stride = (uint32_t)hd.C;
+            }
+            e->pass.gather_samples = std::max(e->pass.gather_samples, (uint32_t)sd.step_batches * B);
+        }
+        if (n_ship)
+            CU(cudaMemcpyAsync(s.d_xfer, s.h_xfer, sizeof(XShip) * n_ship, cudaMemcpyHostToDevice, e->s_in));
+        if (n_gather)
+            CU(cudaMemcpyAsync(s.d_xfer + e->xfer_gather_off, s.h_xfer + e->xfer_gather_off, sizeof(XGather) * n_gather, cudaMemcpyHostToDevice, e->s_in));
+    }
     CU(cudaMemcpyAsync(s.d_desc, s.h_desc, e->desc_bytes, cudaMemcpyHostToDevice, e->s_in));
 
     CU(cudaEventRecord(s.ev_in, e->s_in));
     CU(cudaStreamWaitEvent(e->s_k, s.ev_in, 0));
-
-    /* 3. launches.  The channelizer (FP32/shared-memory bound, fills the SMs) and the demodulator (a latency-bound serial
-     * recurrence, one or two warps per SM) run on two streams: the demodulator of ticket t overlaps the channelizer of
-     * ticket t+1, which writes a disjoint stretch of the pick ring.  With AFC the bins feed back, so one stream is used. */
-    cudaStream_t k2s = e->serial_k2 ? e->s_k : e->s_k2;
-    for (int ph = 0; ph < phases; ph++) {
-        CU(cudaEventRecord(s.ev_k[4 * ph + 0], e->s_k));
-        /* Inputs without AFC never run the instantiation that also writes the spectrum: the two are compiled apart and may
-         * round the FFT differently in the last bit, and an input's audio must not depend on whether another input of its
-         * engine has AFC (nor on which member of a multi-GPU group it was placed in). */
-        for (int afc = 0; afc < 2; afc++) {
-            const int first = afc ? k1_plain[ph] : 0;
-            const int n_dev = afc ? k1_count[ph] - k1_plain[ph] : k1_plain[ph];
-            if (n_dev == 0)
-                continue;
-            K1Params p;
-            p.dev = d_k1 + (size_t)ph * nd + first;
-            p.n_dev = n_dev;
-            p.tile_frames = e->tile_frames;
-            p.n_tiles = afc ? k1_tiles[ph] - k1_plain_tiles[ph] : k1_plain_tiles[ph];
-            p.window = e->d_window;
-            p.twiddle = e->d_twiddle;
-            p.raw_bytes = e->raw_bytes;
-            p.max_channels = e->max_channels;
-            p.tile_counter = e->d_tile_counter;
-            const int ctas = std::min(p.n_tiles, e->sm_count * e->k1_ctas_per_sm);
-            CU(cudaMemsetAsync(e->d_tile_counter, 0, sizeof(uint32_t), e->s_k));
-            int rc = k1_launch(e->fft_size, p, ctas, afc != 0, e->s_k);
+    int rc = launch_k1(e, s, 0);
+    if (rc != BA_OK)
+        return rc;
+    if (!e->ship.empty()) {
+        /* behind K1 of this ticket, once each follower's demodulator of ticket - 2 has let go of the stretch of its pick ring
+         * the ship is about to overwrite */
+        if (ticket >= 2)
+            for (const ShipTo& st : e->ship)
+                CU(cudaStreamWaitEvent(e->s_k, st.to->slot[(ticket - 2) % BA_SLOTS].ev_gather, 0));
+        if (e->pass.n_ship > 0 && e->pass.ship_frames > 0) {
+            rc = x_ship_launch(reinterpret_cast<const XShip*>(s.d_xfer), e->pass.n_ship, e->pass.ship_frames, e->s_k);
             if (rc != 0)
-                return fail(BA_ERR_CUDA, "channelize launch: %s", cudaGetErrorString((cudaError_t)rc));
+                return fail(BA_ERR_CUDA, "ship launch: %s", cudaGetErrorString((cudaError_t)rc));
             e->launches++;
         }
-        CU(cudaEventRecord(s.ev_k[4 * ph + 1], e->s_k));
-        CU(cudaEventRecord(s.ev_k1, e->s_k));
-        if (k2s != e->s_k)
-            CU(cudaStreamWaitEvent(k2s, s.ev_k1, 0));
-        CU(cudaEventRecord(s.ev_k[4 * ph + 2], k2s));
-        if (k2_any[ph]) {
-            K2Params p;
-            p.chan = e->d_chan;
-            p.state = e->d_state;
-            p.dyn = d_dyn + (size_t)ph * nd;
-            p.order = e->d_order;
-            p.n_channels = e->total_channels;
-            p.wave_batch = B;
-            p.sincos = e->d_sincos;
-            int rc = k2_launch(p, e->n_plain, e->sm_count, k2s, e->s_k2b, e->ev_fork, e->ev_join);
-            if (rc != 0)
-                return fail(BA_ERR_CUDA, "demod launch: %s", cudaGetErrorString((cudaError_t)rc));
-            e->launches += (e->n_plain > 0 ? 1 : 0) + (e->total_channels > e->n_plain ? 1 : 0);
-        }
-        CU(cudaEventRecord(s.ev_k[4 * ph + 3], k2s));
+        CU(cudaEventRecord(s.ev_ship, e->s_k));
     }
-    s.phases = phases;
+    return BA_OK;
+}
+
+/* 3: K2 of the first phase, the other phases (K1 + K2 each, AFC inputs), gather.  The channelizer (FP32/shared-memory
+ * bound, fills the SMs) and the demodulator (a latency-bound serial recurrence, one or two warps per SM) run on two streams:
+ * the demodulator of ticket t overlaps the channelizer of ticket t+1, which writes a disjoint stretch of the pick ring.
+ * With AFC the bins feed back, so one stream is used. */
+static int stage_k2(ba_engine* e) {
+    using namespace ba;
+    USE_DEVICE(e);
+    const int ticket = e->pass.ticket;
+    Slot& s = e->slot[ticket % BA_SLOTS];
+    int rc = launch_k2(e, s, 0);
+    for (int ph = 1; ph < e->pass.phases && rc == BA_OK; ph++) {
+        rc = launch_k1(e, s, ph);
+        if (rc == BA_OK)
+            rc = launch_k2(e, s, ph);
+    }
+    if (rc != BA_OK || e->gather.empty())
+        return rc;
+    /* into the homes' result slots, once their device->host copies of ticket - 3 (same slot) have read them */
+    cudaStream_t k2s = e->serial_k2 ? e->s_k : e->s_k2;
+    for (const GatherTo& gt : e->gather)
+        if (gt.home->slot[ticket % BA_SLOTS].used)
+            CU(cudaStreamWaitEvent(k2s, gt.home->slot[ticket % BA_SLOTS].ev_done, 0));
+    if (e->pass.n_gather > 0 && e->pass.gather_samples > 0) {
+        rc = x_gather_launch(reinterpret_cast<const XGather*>(s.d_xfer + e->xfer_gather_off), e->pass.n_gather, e->pass.gather_samples, k2s);
+        if (rc != 0)
+            return fail(BA_ERR_CUDA, "gather launch: %s", cudaGetErrorString((cudaError_t)rc));
+        e->launches++;
+    }
+    CU(cudaEventRecord(s.ev_gather, k2s));
+    return BA_OK;
+}
+
+/* 4: mixers, silent-row packing, results to pinned host memory */
+static int stage_out(ba_engine* e) {
+    using namespace ba;
+    USE_DEVICE(e);
+    const int ticket = e->pass.ticket;
+    Slot& s = e->slot[ticket % BA_SLOTS];
+    const size_t nd = e->dev.size();
+    const int B = e->B;
+    cudaStream_t k2s = e->serial_k2 ? e->s_k : e->s_k2;
+    const int mix_max_emit = e->pass.mix_max_emit, mix_max_stash = e->pass.mix_max_stash;
+    for (const ShipTo& st : e->ship) /* the rows demodulated elsewhere are in place */
+        CU(cudaStreamWaitEvent(k2s, st.to->slot[ticket % BA_SLOTS].ev_gather, 0));
+    s.phases = e->pass.phases;
     if (mix_max_emit > 0 || mix_max_stash > 0) {
         K3Params p;
         p.in = e->d_mix_in;
-        p.in_dyn = d_in_dyn;
+        p.in_dyn = e->pass.d_in_dyn;
         p.mixer = e->d_mixer;
-        p.mix_dyn = d_mix_dyn;
+        p.mix_dyn = e->pass.d_mix_dyn;
         p.fifo = e->d_fifo;
         p.fifo_sig = e->d_fifo_sig;
         p.fifo_depth = e->fifo_depth;
@@ -1701,7 +2117,8 @@ int ba_cuda_process(ba_engine* e) {
     if (skip_silence) {
         uint32_t rows = 0, ch0 = 0;
         int n = 0;
-        for (Dev* d : e->dev) {
+        for (int di = 0; di < e->n_own; di++) { /* a member's shadows go back to their homes */
+            const Dev* d = e->dev[di];
             if (d->step_batches > 0) {
                 s.h_packdev[n].first_channel = ch0;
                 s.h_packdev[n].n_channels = (uint32_t)d->C;
@@ -1726,11 +2143,12 @@ int ba_cuda_process(ba_engine* e) {
     CU(cudaStreamWaitEvent(e->s_out, s.ev_kdone, 0));
     CU(cudaEventRecord(s.ev_out0, e->s_out));
 
-    /* 4. results to pinned host memory */
+    /* 4. results to pinned host memory (a member's shadows, the last of its devices, go back to their homes by gather) */
     {
+        const std::vector<Dev*> own(e->dev.begin(), e->dev.begin() + e->n_own);
         bool uniform = true;
-        int nb0 = e->dev[0]->step_batches;
-        for (Dev* d : e->dev)
+        int nb0 = own.empty() ? 0 : own[0]->step_batches;
+        for (Dev* d : own)
             uniform = uniform && d->step_batches == nb0;
         auto copy_rows = [&](size_t off, size_t rows, int nb) -> int {
             const size_t width = (size_t)nb * B;
@@ -1748,12 +2166,12 @@ int ba_cuda_process(ba_engine* e) {
         } else if (skip_silence) {
             /* the row map and the number of packed rows now; the rows themselves when ba_cuda_collect() knows how many there are */
             if (s.pack_pending) {
-                const size_t rows = (size_t)e->total_channels * e->max_batches;
+                const size_t rows = (size_t)e->own_channels * e->max_batches;
                 CU(cudaMemcpyAsync(s.h_rowmap, s.d_rowmap, sizeof(int32_t) * rows, cudaMemcpyDeviceToHost, e->s_out));
                 CU(cudaMemcpyAsync(s.h_rowcount, s.d_rowcount, sizeof(uint32_t), cudaMemcpyDeviceToHost, e->s_out));
                 s.d2h_bytes += sizeof(int32_t) * rows + sizeof(uint32_t);
                 if (s.d_trace) {
-                    for (Dev* d : e->dev)
+                    for (Dev* d : own)
                         if (d->step_batches > 0) {
                             const size_t width = (size_t)d->step_batches * B;
                             CU(cudaMemcpy2DAsync(s.h_trace + d->wave_off, e->stride, s.d_trace + d->wave_off, e->stride, width, (size_t)d->C, cudaMemcpyDeviceToHost, e->s_out));
@@ -1764,25 +2182,25 @@ int ba_cuda_process(ba_engine* e) {
         } else if (uniform && nb0 == e->max_batches && !s.d_trace) {
             /* a full step everywhere: one linear copy of the arena (the E carried-over samples per row ride along, 1 %) */
             size_t floats = 0;
-            for (Dev* d : e->dev)
+            for (Dev* d : own)
                 floats += (size_t)d->C * e->stride;
             CU(cudaMemcpyAsync(s.h_wave, s.d_wave, sizeof(float) * floats, cudaMemcpyDeviceToHost, e->s_out));
             s.d2h_bytes += sizeof(float) * floats;
         } else if (uniform) {
             if (nb0 > 0) {
-                int rc = copy_rows(0, (size_t)e->total_channels, nb0);
+                int rc = copy_rows(0, (size_t)e->own_channels, nb0);
                 if (rc != BA_OK)
                     return rc;
             }
         } else {
-            for (Dev* d : e->dev)
+            for (Dev* d : own)
                 if (d->step_batches > 0) {
                     int rc = copy_rows(d->wave_off, (size_t)d->C, d->step_batches);
                     if (rc != BA_OK)
                         return rc;
                 }
         }
-        for (Dev* d : e->dev) {
+        for (Dev* d : own) {
             if (d->step_batches <= 0 || !to_host)
                 continue;
             if (s.d_iq && d->any_iq) {
@@ -1793,11 +2211,11 @@ int ba_cuda_process(ba_engine* e) {
             }
         }
         bool any = false;
-        for (Dev* d : e->dev)
+        for (Dev* d : own)
             any = any || d->step_batches > 0;
         if (any) {
             size_t total_status = 0;
-            for (Dev* d : e->dev)
+            for (Dev* d : own)
                 total_status += (size_t)d->C * e->max_batches;
             CU(cudaMemcpyAsync(s.h_status, s.d_status, sizeof(ba_channel_status) * total_status, cudaMemcpyDeviceToHost, e->s_out));
             s.d2h_bytes += sizeof(ba_channel_status) * total_status;
@@ -1823,6 +2241,53 @@ int ba_cuda_process(ba_engine* e) {
     s.used = true;
     e->next_ticket++;
     return ticket;
+}
+
+
+/* a follower's shadow of a split input runs the step its home planned */
+static void copy_shadow_plans(ba_engine* m) {
+    for (const GatherTo& gt : m->gather) {
+        Dev& sd = *m->dev[gt.shadow];
+        const Dev& hd = *gt.home->dev[gt.dev];
+        sd.step_frame0 = hd.step_frame0;
+        sd.step_frames = hd.step_frames;
+        sd.step_batch0 = hd.step_batch0;
+        sd.step_batches = hd.step_batches;
+    }
+}
+
+int ba_cuda_process(ba_engine* e) {
+    if (!e)
+        return fail(BA_ERR_BAD_ARG, "null engine");
+    if (e->members.empty()) {
+        int rc = stage_plan(e);
+        if (rc >= 0)
+            rc = stage_k1(e);
+        if (rc >= 0)
+            rc = stage_k2(e);
+        return rc >= 0 ? stage_out(e) : rc;
+    }
+    /* every member's pass, stage by stage; their tickets move in lockstep */
+    int ticket = -1;
+    int rc = each_member(e, [&](ba_engine* m) {
+        const int t = stage_plan(m);
+        if (t >= 0 && ticket >= 0 && t != ticket)
+            return fail(BA_ERR_STATE, "member tickets %d and %d differ", ticket, t);
+        ticket = t;
+        return t;
+    });
+    if (rc >= 0) {
+        for (ba_engine* m : e->members)
+            copy_shadow_plans(m);
+        rc = each_member(e, stage_k1);
+    }
+    if (rc >= 0)
+        rc = each_member(e, stage_k2);
+    if (rc >= 0)
+        rc = each_member(e, stage_out);
+    if (rc < 0)
+        e->broken = true;
+    return rc < 0 ? rc : ticket;
 }
 
 static Slot* find_slot(ba_engine* e, int ticket) {
@@ -1912,7 +2377,7 @@ int ba_cuda_mixer_input_mask(ba_engine* e, int mixer, int input, int enabled) {
 }
 
 int ba_cuda_set_freq_idx(ba_engine* e, int dev, int channel, int freq_idx, uint64_t* from_batch) {
-    FORWARD_DEV(e, dev, ba_cuda_set_freq_idx(e, dev, channel, freq_idx, from_batch));
+    FORWARD_CHAN(e, dev, channel, ba_cuda_set_freq_idx(e, dev, channel, freq_idx, from_batch));
     Dev* d = get_dev(e, dev);
     if (!d)
         return BA_ERR_BAD_ARG;
@@ -2056,7 +2521,7 @@ int ba_cuda_mark_ms(ba_engine* e, int from, int to, float* ms) {
 }
 
 int ba_cuda_channel_info(ba_engine* e, int dev, int channel, ba_channel_info* out) {
-    FORWARD_DEV(e, dev, ba_cuda_channel_info(e, dev, channel, out));
+    FORWARD_CHAN(e, dev, channel, ba_cuda_channel_info(e, dev, channel, out));
     Dev* d = get_dev(e, dev);
     if (!d || !out || channel < 0 || channel >= d->C)
         return fail(BA_ERR_BAD_ARG, "bad argument");
@@ -2205,6 +2670,30 @@ int ba_cuda_debug_picks(ba_engine* e, int dev, int channel, uint64_t first, int 
 }
 
 int ba_cuda_debug_inject_picks(ba_engine* e, int dev, const float* picks, int n_frames) {
+    if (e && !e->members.empty() && dev >= 0 && dev < (int)e->ch_member.size() && !e->ch_member[dev].empty() && !e->broken && picks && n_frames >= 0) {
+        /* a split input: the home takes every channel, as K1 would have written them; each follower's shadow the columns
+         * of its channels, as the ship would have */
+        ba_engine* g = e;
+        const int C = (int)g->ch_member[dev].size();
+        int rc = group_rc(g, ba_cuda_debug_inject_picks(g->members[g->dev_member[dev]], g->dev_local[dev], picks, n_frames));
+        if (rc != BA_OK)
+            return rc;
+        for (const ShipTo& st : g->members[g->dev_member[dev]]->ship) {
+            if (st.dev != g->dev_local[dev])
+                continue;
+            const size_t n = st.home_ch.size();
+            std::vector<float> sub((size_t)n_frames * n * 2);
+            for (size_t f = 0; f < (size_t)n_frames; f++)
+                for (size_t k = 0; k < n; k++) {
+                    sub[2 * (f * n + k)] = picks[2 * (f * C + st.home_ch[k])];
+                    sub[2 * (f * n + k) + 1] = picks[2 * (f * C + st.home_ch[k]) + 1];
+                }
+            rc = group_rc(g, ba_cuda_debug_inject_picks(st.to, st.shadow, sub.data(), n_frames));
+            if (rc != BA_OK)
+                return rc;
+        }
+        return BA_OK;
+    }
     FORWARD_DEV(e, dev, ba_cuda_debug_inject_picks(e, dev, picks, n_frames));
     Dev* d = get_dev(e, dev);
     if (!d || !picks || n_frames < 0)

@@ -218,5 +218,34 @@ int k3_pack_launch(const K3PackDev* devs, int n_dev, int total_rows, const float
 /* mixes max_emit (largest n_emit of any mixer) batches, then parks max_stash (largest stash_count) */
 int k3_launch(const K3Params& p, int n_mixers, int max_emit, int n_inputs, int max_stash, cudaStream_t s);
 
+/* ------------------------------------------------------------------ channel sharding (mixer.cu) */
+/* An input whose channels are demodulated on several GPUs is channelized once, on its home GPU.  Both kernels store to the
+ * other GPU's memory (peer stores; a plain store when both sides share one GPU).  Their job tables live in device memory. */
+
+/* ship (on the home, behind K1): one channel's magnitudes, and its picked IQ where the follower reads it, for the frames the
+ * home channelized in this step, from the home's pick ring to the same ring positions of the follower's */
+struct XShip {
+    const float* src_mags;
+    float* dst_mags;          /* rows of [ring_len] */
+    const float2* src_picks;
+    float2* dst_picks;        /* NULL: the IQ stays home */
+    uint64_t frame0;          /* first frame of the step */
+    uint32_t n_frames, ring_mask;
+};
+/* gather (on the follower, behind K2): one channel's results of the step into the home's result slot */
+struct XGather {
+    const float* src_wave;
+    float* dst_wave;          /* n_samples floats */
+    const uint8_t* src_trace;
+    uint8_t* dst_trace;       /* or NULL */
+    const float2* src_iq;
+    float2* dst_iq;           /* or NULL */
+    const ba_channel_status* src_status;
+    ba_channel_status* dst_status; /* &status[0][channel] */
+    uint32_t n_samples, n_batches, src_status_stride, dst_status_stride; /* strides in entries between batches */
+};
+int x_ship_launch(const XShip* jobs, int n_jobs, uint32_t max_frames, cudaStream_t s);
+int x_gather_launch(const XGather* jobs, int n_jobs, uint32_t max_samples, cudaStream_t s);
+
 }  // namespace ba
 #endif

@@ -35,6 +35,21 @@
 static inline unsigned atomicAdd(unsigned* p, unsigned v) {
     return __atomic_fetch_add(p, v, __ATOMIC_RELAXED);
 }
+/* peer access between emulated devices (one address space: every pair can reach each other).  BA_EMU_NO_PEER set to a
+ * non-zero value makes cudaDeviceCanAccessPeer answer 0, so that a test can see the engine refuse a GPU pair without it. */
+enum { cudaErrorPeerAccessAlreadyEnabled = 704 };
+static inline cudaError_t cudaDeviceCanAccessPeer(int* can, int d, int peer) {
+    const char* v = getenv("BA_EMU_NO_PEER");
+    if (d < 0 || d >= emu::device_count() || peer < 0 || peer >= emu::device_count())
+        return cudaErrorInvalidValue;
+    *can = (d != peer && !(v && atoi(v) != 0)) ? 1 : 0;
+    return cudaSuccess;
+}
+static inline cudaError_t cudaDeviceEnablePeerAccess(int peer, unsigned) {
+    if (peer < 0 || peer >= emu::device_count() || peer == emu::current_device())
+        return cudaErrorInvalidValue;
+    return cudaSuccess;
+}
 static inline unsigned __byte_perm(unsigned x, unsigned y, unsigned s) {
     const unsigned long long src = ((unsigned long long)y << 32) | x;
     unsigned r = 0;

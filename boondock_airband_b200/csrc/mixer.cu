@@ -12,6 +12,9 @@
  *
  * Compiled with -fmad=false: the product and the sum round separately, as the reference's C does.
  * HBM-bound elementwise work: 4 bytes read per input sample with signal, 4 (8 stereo) written per output sample.
+ *
+ * Also here: ship_kernel and gather_kernel, the copies between the members of a group that spreads one input's channels
+ * over several GPUs (ba_cuda_create_multi_split, DESIGN.md section 6).
  */
 #include "ba_kernels.h"
 
@@ -150,7 +153,60 @@ __global__ void __launch_bounds__(256) pack_rows_kernel(const K3PackDev* devs, i
         rowmap[(size_t)ch * max_batches + b] = slot;
 }
 
+/* channel sharding: HBM/NVLink-bound copies, one CTA row per job, threads over the frames (samples) of the step */
+__global__ void __launch_bounds__(256) ship_kernel(const XShip* jobs, int n_jobs) {
+    for (int jb = blockIdx.y; jb < n_jobs; jb += gridDim.y) {
+        const XShip j = jobs[jb];
+        for (uint32_t i = blockIdx.x * 256 + threadIdx.x; i < j.n_frames; i += gridDim.x * 256) {
+            const uint32_t pos = (uint32_t)((j.frame0 + i) & (uint64_t)j.ring_mask);
+            j.dst_mags[pos] = j.src_mags[pos];
+            if (j.dst_picks)
+                j.dst_picks[pos] = j.src_picks[pos];
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) gather_kernel(const XGather* jobs, int n_jobs) {
+    for (int jb = blockIdx.y; jb < n_jobs; jb += gridDim.y) {
+        const XGather j = jobs[jb];
+        const uint32_t t0 = blockIdx.x * 256 + threadIdx.x, step = gridDim.x * 256;
+        for (uint32_t i = t0; i < j.n_samples; i += step) {
+            j.dst_wave[i] = j.src_wave[i];
+            if (j.dst_trace)
+                j.dst_trace[i] = j.src_trace[i];
+            if (j.dst_iq)
+                j.dst_iq[i] = j.src_iq[i];
+        }
+        const uint32_t words = (uint32_t)(sizeof(ba_channel_status) / 4);
+        for (uint32_t i = t0; i < j.n_batches * words; i += step) {
+            const uint32_t b = i / words, w = i % words;
+            reinterpret_cast<uint32_t*>(j.dst_status + (size_t)b * j.dst_status_stride)[w] =
+                reinterpret_cast<const uint32_t*>(j.src_status + (size_t)b * j.src_status_stride)[w];
+        }
+    }
+}
+
+/* CTAs per job along the frames / samples: enough to cover a short step in one pass, few enough that a long one loops */
+inline unsigned x_blocks(uint32_t n) {
+    const unsigned b = (n + 255) / 256;
+    return b < 1 ? 1 : (b > 8 ? 8 : b);
+}
+
 }  // namespace
+
+int x_ship_launch(const XShip* jobs, int n_jobs, uint32_t max_frames, cudaStream_t s) {
+    if (n_jobs <= 0 || max_frames == 0)
+        return 0;
+    BA_LAUNCH(ship_kernel, dim3(x_blocks(max_frames), n_jobs < 65535 ? n_jobs : 65535), 256, 0, s, jobs, n_jobs);
+    return (int)cudaGetLastError();
+}
+
+int x_gather_launch(const XGather* jobs, int n_jobs, uint32_t max_samples, cudaStream_t s) {
+    if (n_jobs <= 0 || max_samples == 0)
+        return 0;
+    BA_LAUNCH(gather_kernel, dim3(x_blocks(max_samples), n_jobs < 65535 ? n_jobs : 65535), 256, 0, s, jobs, n_jobs);
+    return (int)cudaGetLastError();
+}
 
 int k3_pack_launch(const K3PackDev* devs, int n_dev, int total_rows, const float* wave, int stride, int wave_batch, float* pack, int32_t* rowmap, int max_batches,
                    uint32_t* count, cudaStream_t s) {

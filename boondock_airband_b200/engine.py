@@ -30,7 +30,7 @@ SYMBOLS = (
     "ba_cuda_advance_device_stream", "ba_cuda_process", "ba_cuda_collect", "ba_cuda_collect_mixer", "ba_cuda_mixer_input_mask", "ba_cuda_set_freq_idx", "ba_cuda_ticket_ms", "ba_cuda_step_bytes",
     "ba_cuda_channel_info", "ba_cuda_window", "ba_cuda_debug_frames", "ba_cuda_debug_picks",
     "ba_cuda_debug_inject_picks", "ba_cuda_launch_count", "ba_cuda_kernel_ms", "ba_cuda_copy_ms", "ba_cuda_mark", "ba_cuda_mark_ms",
-    "ba_cuda_create_multi", "ba_cuda_device_gpu",
+    "ba_cuda_create_multi", "ba_cuda_device_gpu", "ba_cuda_create_multi_split", "ba_cuda_channel_gpu",
 )
 
 
@@ -54,6 +54,8 @@ def load_library(path: Optional[str] = None):
     i32p = C.POINTER(C.c_int32)
     L.ba_cuda_create_multi.argtypes = [C.POINTER(abi.EngineDesc), i32p, C.c_int32, i32p, C.POINTER(vp)]
     L.ba_cuda_device_gpu.argtypes = [vp, C.c_int, i32p]
+    L.ba_cuda_create_multi_split.argtypes = [C.POINTER(abi.EngineDesc), i32p, C.c_int32, i32p, C.POINTER(i32p), C.POINTER(vp)]
+    L.ba_cuda_channel_gpu.argtypes = [vp, C.c_int, C.c_int, i32p]
     L.ba_cuda_destroy.argtypes = [vp]
     L.ba_cuda_destroy.restype = None
     L.ba_cuda_last_error.restype = C.c_char_p
@@ -164,17 +166,20 @@ def device_to_host(ptr: int, nbytes: int) -> bytes:
 
 class Engine:
     def __init__(self, cfg: abi.EngineCfg, lib_path: Optional[str] = None, gpus: Optional[Sequence[int]] = None,
-                 gpu_of_device: Optional[Sequence[int]] = None):
+                 gpu_of_device: Optional[Sequence[int]] = None, gpu_of_channel: Optional[Sequence[Optional[Sequence[int]]]] = None):
         """One engine on cfg.cuda_device; with ``gpus`` (CUDA ordinals, repeats allowed) one engine over those GPUs
         (ba_cuda_create_multi): devices are placed by ``gpu_of_device`` (indices into gpus) or, without it, with the
-        devices of a mixer kept together and groups dealt out round robin.  Every method works the same either way."""
+        devices of a mixer kept together and groups dealt out round robin.  ``gpu_of_channel`` (one entry per device:
+        None, or per channel an index into gpus) spreads a device's channels over several GPUs
+        (ba_cuda_create_multi_split): the device is channelized at its home, each channel demodulated where it is put.
+        Every method works the same either way."""
         self.cfg = cfg
         self.L = load_library(lib_path)
         desc, self._keep = abi.build_desc(cfg)
         h = C.c_void_p()
         if gpus is None:
-            if gpu_of_device is not None:
-                raise ValueError("gpu_of_device needs gpus")
+            if gpu_of_device is not None or gpu_of_channel is not None:
+                raise ValueError("gpu_of_device and gpu_of_channel need gpus")
             rc = self.L.ba_cuda_create(C.byref(desc), C.byref(h))
             where = "ba_cuda_create"
         else:
@@ -182,8 +187,21 @@ class Engine:
                 raise ValueError("gpu_of_device has %d entries for %d devices" % (len(gpu_of_device), len(cfg.devices)))
             g = (C.c_int32 * max(1, len(gpus)))(*gpus)
             m = None if gpu_of_device is None else (C.c_int32 * max(1, len(gpu_of_device)))(*gpu_of_device)
-            rc = self.L.ba_cuda_create_multi(C.byref(desc), g, len(gpus), m, C.byref(h))
-            where = "ba_cuda_create_multi"
+            if gpu_of_channel is None:
+                rc = self.L.ba_cuda_create_multi(C.byref(desc), g, len(gpus), m, C.byref(h))
+                where = "ba_cuda_create_multi"
+            else:
+                if len(gpu_of_channel) != len(cfg.devices):
+                    raise ValueError("gpu_of_channel has %d entries for %d devices" % (len(gpu_of_channel), len(cfg.devices)))
+                i32p = C.POINTER(C.c_int32)
+                rows = [None if x is None else (C.c_int32 * max(1, len(x)))(*x) for x in gpu_of_channel]
+                for x, dev in zip(gpu_of_channel, cfg.devices):
+                    if x is not None and len(x) != len(dev.channels):
+                        raise ValueError("gpu_of_channel entry has %d indices for %d channels" % (len(x), len(dev.channels)))
+                table = (i32p * len(rows))(*[C.cast(r, i32p) if r is not None else i32p() for r in rows])
+                self._keep = (self._keep, rows, table)
+                rc = self.L.ba_cuda_create_multi_split(C.byref(desc), g, len(gpus), m, table, C.byref(h))
+                where = "ba_cuda_create_multi_split"
         if rc != 0:
             raise EngineError(where, rc, self.L.ba_cuda_last_error().decode())
         self.h = h
@@ -301,6 +319,12 @@ class Engine:
         """CUDA ordinal that device ``dev`` runs on: where its device-resident stream and device results must live."""
         n = C.c_int32()
         self._check("ba_cuda_device_gpu", self.L.ba_cuda_device_gpu(self.h, dev, C.byref(n)))
+        return n.value
+
+    def channel_gpu(self, dev: int, ch: int) -> int:
+        """CUDA ordinal whose demodulator runs channel ``ch`` of device ``dev`` (device_gpu(dev) unless the device is split)."""
+        n = C.c_int32()
+        self._check("ba_cuda_channel_gpu", self.L.ba_cuda_channel_gpu(self.h, dev, ch, C.byref(n)))
         return n.value
 
     def launch_count(self) -> int:

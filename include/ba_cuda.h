@@ -248,6 +248,24 @@ BA_API int ba_cuda_create_multi(const ba_engine_desc* desc, const int32_t* gpus,
 /* The CUDA ordinal device `dev` runs on (a plain engine: its cuda_device).  Memory given to ba_cuda_attach_device_stream()
  * must be on that GPU, and the BA_FLAG_RESULTS_ON_DEVICE pointers of the device point there. */
 BA_API int ba_cuda_device_gpu(ba_engine* e, int dev, int32_t* cuda_ordinal);
+/*
+ * The same group, with the channels of a wideband input spread over several GPUs: channelize once, demodulate everywhere,
+ * gather the results at home.  ba_cuda_create_multi() is this call with gpu_of_channel NULL.
+ *   gpu_of_channel       NULL, or desc->device_count pointers.  A NULL pointer keeps the whole device at its home (where
+ *                        gpu_of_device or the default placement puts it); else it points to the device's channel_count
+ *                        indices into gpus, the GPU whose demodulator runs each channel.
+ * The home receives the input, channelizes all of its bins, runs its mixers and owns the results ba_cuda_collect() hands
+ * out.  Every other GPU named for some of its channels gets their picked bins by peer stores right behind the home's
+ * channelizer, demodulates them, and stores their audio, status, trace and iq_out into the home's result slot of the same
+ * ticket.  The results are bit for bit those of one engine.  ba_cuda_set_freq_idx() and ba_cuda_channel_info() go to the
+ * GPU that runs the channel.  Peer access is enabled between a home and its other GPUs.  BA_ERR_BAD_ARG (beyond those of
+ * ba_cuda_create_multi) for a channel index out of range, a split device with an AFC channel, and a GPU without peer access
+ * to the home in either direction. */
+BA_API int ba_cuda_create_multi_split(const ba_engine_desc* desc, const int32_t* gpus, int32_t n_gpus, const int32_t* gpu_of_device,
+                                      const int32_t* const* gpu_of_channel, ba_engine** out);
+/* The CUDA ordinal whose demodulator runs channel `channel` of device `dev` (an unsplit device or a plain engine: the same as
+ * ba_cuda_device_gpu()). */
+BA_API int ba_cuda_channel_gpu(ba_engine* e, int dev, int channel, int32_t* cuda_ordinal);
 /* Replaces gpu_fft_release (src/boondock_airband.cpp:385-388). */
 BA_API void ba_cuda_destroy(ba_engine* e);
 /* Text of the most recent failure on this thread (never NULL). */
